@@ -90,6 +90,9 @@ def parse_args(argv=None):
     ap.add_argument("--classes", default="all", choices=["all", "all20", "live"],
                     help="all: every image is captioned with every class of the configuration (BASELINE configs); live (config 1): "
                          "classes per image drawn from the reference's own GPT-4o answers for VOC (mean 1.40)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64; rank 0), so "
+                         "that two builds run with the same arguments can be compared output for output")
     a = ap.parse_args(argv)
     if a.classes == "all20":
         a.classes = "all"
@@ -382,6 +385,7 @@ def run_ours(args):
     hist_host = [torch.empty((n_cls, n_cls), dtype=torch.int64).pin_memory() for _ in range(2)]
     d2h_events = []
     bad = torch.zeros(1, dtype=torch.int32, device=dev)
+    last_step = []      # what batch_confusion returned for each batch of the most recent step (--dump-outputs)
     scored = "all_drop" if cfg["drop_iter"] > 1 else "round0"
 
     def run_batch(s, e2e, stats=None, labels_out=None, overlap=None, defer=False):
@@ -401,13 +405,14 @@ def run_ours(args):
         def gradcam_fn(x):
             return model.gradcam(x, wl["captions"], s.tokens_dev, layer=cfg["layer"], head=cfg["head"])[0]
 
-        h0, hagg, _ = pipeline.batch_confusion(gradcam_fn, s.imgs_d, s.token_ids, wl["tok"].decode, wl["class_lists"], wl["dataset_ids"],
-                                               s.gts_d[i], s.guides_d[i], drop_iter=cfg["drop_iter"], patch_num=cfg["P"],
-                                               threshold=cfg["threshold"], data_type=cfg["data_type"], mode=cfg["mode"], coco=cfg["coco"],
-                                               n_class=n_cls, stats=stats, overlap=(not args.no_overlap) if overlap is None else overlap,
-                                               labels_out=labels_out, bad_count=bad, defer=defer)
+        h0, hagg, chosen = pipeline.batch_confusion(gradcam_fn, s.imgs_d, s.token_ids, wl["tok"].decode, wl["class_lists"], wl["dataset_ids"],
+                                                    s.gts_d[i], s.guides_d[i], drop_iter=cfg["drop_iter"], patch_num=cfg["P"],
+                                                    threshold=cfg["threshold"], data_type=cfg["data_type"], mode=cfg["mode"], coco=cfg["coco"],
+                                                    n_class=n_cls, stats=stats, overlap=(not args.no_overlap) if overlap is None else overlap,
+                                                    labels_out=labels_out, bad_count=bad, defer=defer)
         if defer and e2e:
             s.free_ev[i] = side.record_event()
+        last_step.append({"hist_round0": h0, "hist_all_drop": hagg, "dropout_chosen": chosen})
         return h0, (hagg if hagg is not None else h0)
 
     def step(e2e, stats=None, serial=False, mode=None):
@@ -420,6 +425,7 @@ def run_ours(args):
             serial, defer = mode == "serial", mode == "pipelined"
         else:
             defer = pipelined and stats is None and not serial
+        del last_step[:]
         for s in slots:
             _, h = run_batch(s, e2e, stats, defer=defer, overlap=False if serial else (True if mode is not None else None))
             if defer:
@@ -512,6 +518,7 @@ def run_ours(args):
     lib.pnp_profile_filter_stream(ctypes.c_void_p(side.cuda_stream if pipelined else torch.cuda.current_stream().cuda_stream), 1)
     lib.pnp_profile_start(ctypes.c_uint(1 << dom_id))
     ms_total, reduced = timed(False, args.steps)
+    timed_outputs = list(last_step)
     lib.pnp_profile_stop(tot, cnt, n_ids)
     lib.pnp_profile_filter_stream(ctypes.c_void_p(0), 0)
     clocks = sampler.stop()
@@ -549,6 +556,8 @@ def run_ours(args):
     if int(bad.item()):
         raise SystemExit("bench.py: a relabelled id fell outside [0, n_class)")
     model.check_fp16_overflow()      # 3xFP16 operands: raised if an activation ever left fp16's range (never read per step)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, timed_outputs, reduced)
 
     # ---- multi-GPU: rank 0 recomputes every rank's shard itself and compares with the all-reduced matrix, bit for bit
     allreduce_check = None
@@ -697,6 +706,21 @@ def run_ours(args):
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, batches, reduced):
+    """--dump-outputs: each array batch_confusion returned in the last timed step, the batches of the step stacked on a leading
+    axis (hist_round0 / hist_all_drop [batches, n_class, n_class], dropout_chosen [batches, B, 10 * drop_iter]; an array the
+    configuration does not produce is not written), and hist_timed_total, the confusion matrix summed over every timed step and
+    rank.  float64 holds the int64 counts and the patch indices exactly; the largest case (configs[3], strong scaling) writes
+    under 3 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"hist_timed_total": reduced}
+    for name, first in batches[0].items():
+        if first is not None:
+            arrays[name] = torch.stack([b[name] for b in batches])
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float64))
 
 
 def parity_leg(cfg, slot, run_batch, n_images=4):

@@ -30,10 +30,11 @@ def case_inputs(tag):
     else:
         ids = [[VOC_NMS.index(c) + 1 for c in cl] for cl in class_lists]
         n_class = n_cats + 1
+    B = len(class_lists)   # the cases share one set of inputs; a case of B images takes the first B
     return dict(coco=coco, data_type=data_type, class_lists=class_lists, R=R, S=S, P=P, H=H, W=W, T=T, n_class=n_class,
                 tok=tok, tokens=tt, rows=torch.from_numpy(g["drv_%s_rows" % tag]),
-                imgs=torch.from_numpy(g["drv_%s_imgs" % tag]), gts=list(g["drv_%s_gt" % tag]),
-                guides=list(g["drv_%s_guide" % tag]), ids=ids, golden=g)
+                imgs=torch.from_numpy(g["drv_imgs"][:B].copy()), gts=list(g["drv_gt"][:B]),
+                guides=list(g["drv_guide"][:B]), ids=ids, golden=g)
 
 
 def run_oracle(tag, mode):

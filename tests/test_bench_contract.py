@@ -124,6 +124,43 @@ def test_reference_arm_prints_the_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_dump_outputs_writes_the_last_step_as_float64(tmp_path):
+    """--dump-outputs: one .npy per array batch_confusion returns, batches stacked, values exact; absent arrays are not written."""
+    import torch
+    assert bench.parse_args([]).dump_outputs is None
+    assert bench.parse_args(["--dump-outputs", str(tmp_path)]).dump_outputs == str(tmp_path)
+    h = [torch.arange(9, dtype=torch.int64).view(3, 3) * (k + 1) for k in range(2)]
+    chosen = [torch.full((4, 40), k - 1, dtype=torch.int32) for k in range(2)]
+    batches = [{"hist_round0": None, "hist_all_drop": h[k], "dropout_chosen": chosen[k]} for k in range(2)]
+    bench.dump_outputs(str(tmp_path / "out"), batches, h[0] + h[1])
+    assert sorted(os.listdir(tmp_path / "out")) == ["dropout_chosen.npy", "hist_all_drop.npy", "hist_timed_total.npy"]
+    got = {n: np.load(tmp_path / "out" / (n + ".npy")) for n in ("dropout_chosen", "hist_all_drop", "hist_timed_total")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert np.array_equal(got["hist_all_drop"], torch.stack(h).numpy()) and np.array_equal(got["hist_timed_total"], (h[0] + h[1]).numpy())
+    assert np.array_equal(got["dropout_chosen"], torch.stack(chosen).numpy())
+
+
+@pytest.mark.gpu
+def test_our_arm_times_the_requested_steps_and_dumps_the_last_one(tmp_path):
+    """configs[0] (one image, drop_iter 1) end to end through bench.py: --steps sets the timed steps, and the dumped matrix of the
+    last step times the step count is the matrix accumulated over the timed region."""
+    import json
+    import subprocess
+    import torch
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "0", "--steps", "2", "--warmup", "0",
+                        "--no-cpu-baseline", "--no-e2e", "--no-alt", "--no-parity", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert d["steps"] == 2 and d["hist_total"] == d["hist_expected"]
+    assert sorted(os.listdir(tmp_path)) == ["hist_round0.npy", "hist_timed_total.npy"]   # drop_iter 1: no DropOut outputs
+    h0, total = np.load(tmp_path / "hist_round0.npy"), np.load(tmp_path / "hist_timed_total.npy")
+    assert h0.shape == (1, 21, 21) and h0.dtype == np.float64
+    assert h0.sum() * 2 == d["hist_expected"] and np.array_equal(h0[0] * 2, total)
+
+
 def test_our_arm_refuses_to_run_without_a_gpu():
     """No CPU fallback: on a box without CUDA the product arm of bench.py stops with a clear message (and exit code != 0)."""
     import subprocess

@@ -91,10 +91,11 @@ def _run_driver_case(golden, tag, argsort_kind=None):
     tok = synth.SyntheticWordPieceTokenizer()
     caps = ["A picture of " + " ".join(cl) for cl in class_lists]
     tt = tok(caps, padding="max_length", max_length=500)
+    B = len(class_lists)   # the cases share one set of inputs; a case of B images takes the first B
     rows = torch.from_numpy(golden["drv_%s_rows" % tag])
-    imgs = torch.from_numpy(golden["drv_%s_imgs" % tag])
-    gts = list(golden["drv_%s_gt" % tag])
-    guides = list(golden["drv_%s_guide" % tag])
+    imgs = torch.from_numpy(golden["drv_imgs"][:B].copy())
+    gts = list(golden["drv_gt"][:B])
+    guides = list(golden["drv_guide"][:B])
     fn = synth.SynthGradcamFn(31, len(caps), T, P)
     if coco:  # sparse category ids (cats[idx]['id'], DRVC:549-584) and the COCO matrix sizes (DRVC:597-600)
         catids = golden["drv_%s_catids" % tag]
