@@ -14,10 +14,9 @@
  *   - tensors are dense, row-major, fp32 unless stated; shapes are written [outer, ..., inner];
  *   - one process per GPU (DRV:1439 mp.spawn).  Every entry point except pnp_profile_* may be called from several host threads
  *     at once, each on its own stream (pipeline.py issues the buckets of a ragged batch that way).  Process-global state is limited
- *     to: the in-situ profiler (pnp_profile_*, off by default, single-threaded use only), the per-kernel "allow > 48 KB of dynamic
- *     shared memory" function attribute (granted once per kernel at the device maximum, under a mutex), and tuning environment
- *     variables (PNP_GRID_MULT_*, PNP_BLUR_FUSE*, PNP_UPDATE_*, PNP_VALUE_PITCH, PNP_SPLAT_ATOMIC, PNP_ATT_VARIANT read once,
- *     PNP_ATT_TCGEN05 read per call: experiment switches, unset in production).  No data is cached between calls.
+ *     to: the in-situ profiler (pnp_profile_*, off by default, single-threaded use only) and the per-kernel "allow > 48 KB of
+ *     dynamic shared memory" function attribute (granted once per kernel at the device maximum, under a mutex).  The library reads
+ *     no environment variables.  No data is cached between calls.
  *   - exception to "returns immediately": pnp_lattice_finish synchronises the stream (it reads the vertex count back).
  */
 #ifndef PNP_OVSS_B200_H
@@ -280,8 +279,9 @@ int pnp_layernorm_fp16_split3(const float *x, const float *residual, float resid
 /* Encoder self-attention softmax(Q K^T * softmax_scale) V (VIT:93-119) at fp32-grade accuracy on the fp16 tensor cores: every
  * operand split as above, each product as three fp16 products with fp32 accumulation (main term and corrections apart), online
  * softmax in fp32; nothing of size L x L touches HBM.  The main kernel issues tcgen05.mma with its accumulators in tensor memory
- * (csrc/attention_tc5.cu); the environment variable PNP_ATT_TCGEN05=0 (read per call) selects the mma.sync kernel instead.  qkv [B,L,3,H,D] fp32 exactly as the fused qkv GEMM leaves it (each value
- * times 1/in_scale, in_scale a power of two; 1 for a plain projection); out [B,L,H*D] fp32, unscaled.  D must be 64. */
+ * (csrc/attention.cu).  qkv [B,L,3,H,D] fp32 exactly as the fused qkv GEMM leaves it (each value times 1/in_scale, in_scale a
+ * power of two; 1 for a plain projection); out [B,L,H*D] fp32, unscaled.  D must be 64.  The workspace holds the fp16 (hi, lo)
+ * split of k and v. */
 size_t pnp_attention_fp16x3_workspace_bytes(int B, int L, int H, int D);
 /* out and / or out3 (at least one): out3 [B*L, 3*H*D] fp16 is the [h * out3_hi_scale | l | h] operand split of the output
  * (pnp_fp16_split3's layout), written straight from the accumulators for the projection GEMM that follows. */

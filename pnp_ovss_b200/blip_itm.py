@@ -113,14 +113,11 @@ def _mm16(x16, w16):
     return torch.mm(x16.reshape(-1, x16.shape[-1]), w16.t(), out_dtype=torch.float32).view(*x16.shape[:-1], w16.shape[0])
 
 
-MM3_SEPARATE_CORRECTION = True
-
-
 def _mm3(x3, w3, bias=None):
     """y = x W^T (+ bias) at fp32-grade accuracy on the TF32 tensor cores over the tripled operands (fp32 accumulate; the
     dropped x_lo W_lo term is ~2^-22 relative).  Still plain torch dense contractions (cuBLAS).
 
-    Two launches by default: the main product x_hi W_hi^T (depth K), then the two correction products accumulated onto it
+    Two launches: the main product x_hi W_hi^T (depth K), then the two correction products accumulated onto it
     in place ([x_lo | x_hi] [W_hi | W_lo]^T, depth 2K, beta = 1).  The tensor core adds into its fp32 accumulator with
     truncation, an error that grows with the depth of ONE accumulation chain: keeping the 2^-11-sized corrections out of
     the main chain leaves rms 4.8e-7 of max|y| at K = 1024 (native SIMT fp32: 1.1e-7; all three products in one depth-3K
@@ -128,8 +125,6 @@ def _mm3(x3, w3, bias=None):
     prev = torch.backends.cuda.matmul.allow_tf32
     torch.backends.cuda.matmul.allow_tf32 = True
     try:
-        if not MM3_SEPARATE_CORRECTION:
-            return F.linear(x3, w3, bias)
         K = w3.shape[1] // 3
         x2 = x3.reshape(-1, 3 * K)
         y = F.linear(x2[:, :K], w3[:, :K], bias)
@@ -139,35 +134,21 @@ def _mm3(x3, w3, bias=None):
         torch.backends.cuda.matmul.allow_tf32 = prev
 
 
-def _mm3_single(x3, w3, bias=None):
-    """The three products in ONE depth-3K TF32 GEMM (one launch; used for the small text-side GEMMs, which are launch-bound)."""
-    prev = torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cuda.matmul.allow_tf32 = True
-    try:
-        return F.linear(x3, w3, bias)
-    finally:
-        torch.backends.cuda.matmul.allow_tf32 = prev
-
-
 class _Linear3(torch.autograd.Function):
     """y = x W^T + b for a FROZEN weight on the TF32 tensor cores at fp32 grade (exact hi/lo split, three products), forward and
     backward: dL/dx = dL/dy W is the same kind of product against the split of W^T.  TF32 keeps fp32's exponent range, so the
     tiny gradients of the trimmed backward (1e-6 and below) lose nothing -- which is why the text side does not use fp16."""
 
-    SINGLE_GEMM = False   # True: all three products in one depth-3K GEMM (one launch per linear instead of two)
-
     @staticmethod
     def forward(ctx, x, w3, wt3, bias):
         ctx.wt3 = wt3
         ctx.x_shape = x.shape
-        mm = _mm3_single if _Linear3.SINGLE_GEMM else _mm3
-        y = mm(ops.tf32_split3(x.reshape(-1, x.shape[-1]).contiguous()), w3, bias)
+        y = _mm3(ops.tf32_split3(x.reshape(-1, x.shape[-1]).contiguous()), w3, bias)
         return y.view(*x.shape[:-1], w3.shape[0])
 
     @staticmethod
     def backward(ctx, gy):
-        mm = _mm3_single if _Linear3.SINGLE_GEMM else _mm3
-        gx = mm(ops.tf32_split3(gy.reshape(-1, gy.shape[-1]).contiguous()), ctx.wt3)
+        gx = _mm3(ops.tf32_split3(gy.reshape(-1, gy.shape[-1]).contiguous()), ctx.wt3)
         return gx.view(ctx.x_shape), None, None, None
 
 
@@ -472,7 +453,7 @@ class BlipITM(nn.Module):
             # the attention's scale (2^-22 / sqrt(d)) and the next split (2^-11) take back exactly
             qkv = mm(h3, w_qkv[0]) if half else _mm3(h3, w_qkv[0], blk.qkv.bias)
             hd = D // blk.heads
-            if half and self.USE_FUSED_ATTENTION and hd == 64:
+            if half and hd == 64:
                 # the attention itself on the fp16 tensor cores with the same hi/lo split (pnp_attention_fp16x3): unscaled output
                 a3 = ops.attention_fp16x3(qkv.view(B, L, 3, blk.heads, hd), inv, 1.0 / math.sqrt(hd), flag, split_hi_scale=w_proj[1])
                 r = mm(a3, w_proj[0])
@@ -517,7 +498,6 @@ class BlipITM(nn.Module):
         return [(kv[:, :, i, 0], kv[:, :, i, 1], s) for i in range(n)]
 
     USE_VIT_GRAPH = True
-    USE_FUSED_ATTENTION = True     # 3xfp16 mode: encoder attention through pnp_attention_fp16x3 instead of torch's fp32 SDPA
 
     def _encode(self, imgs):
         """(enc or None, per-block cross-attention (k, v) or [None]*n) for the current gemm_precision."""

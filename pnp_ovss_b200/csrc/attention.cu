@@ -1,51 +1,36 @@
-// attention.cu -- ViT self-attention softmax(Q K^T / sqrt(d)) V at fp32-grade accuracy on the fp16 tensor cores (VIT:93-119, the
-// attention of every encoder block; SURVEY 8f.1: the model pass).
+// attention.cu -- ViT self-attention softmax(Q K^T / sqrt(d)) V at fp32-grade accuracy on the 5th-generation tensor cores (tcgen05.mma,
+// accumulators in tensor memory); VIT:93-119, the attention of every encoder block (SURVEY 8f.1: the model pass).
 //
 // Same idea as the 3xFP16 GEMM operands (tf32x3.cu): every fp32 operand is split exactly into x = h + l 2^-11 (h = fp16(x),
-// l = fp16((x - h) 2^11)) and each product a b is evaluated as  a_h b_h + 2^-11 (a_l b_h + a_h b_l)  -- three fp16
-// mma.sync.m16n8k16 with fp32 accumulation, the main term and the two corrections in separate accumulators (the tensor core
-// adds with truncation: the 2^-11-sized corrections must not sit in the main chain).  That holds for both contractions:
-// S = Q K^T and O = P V, with the probabilities P split the same way after the fp32 online softmax.
-// Two passes.  (1) q, k, v are split once into fp16 (hi, lo) pairs in a workspace (q pre-scaled for an exp2 softmax).
-// (2) Flash-attention structure: one CTA = 64 query rows of one (image, head), 4 warps x 16 rows; K and V tiles of 64 keys
-// stream through a double-buffered cp.async pipeline in shared memory; nothing of size L x L touches HBM.
-// HBM traffic: q, k, v read once, their splits written once and read once (K/V tiles hit in L2 across the 7 query tiles of a
-// head), O written once.
+// l = fp16((x - h) 2^11)) and each product a b is evaluated as  a_h b_h + 2^-11 (a_l b_h + a_h b_l)  with fp32 accumulation, the main
+// term and the two corrections in separate accumulators (the tensor core adds with truncation: the 2^-11-sized corrections must not
+// sit in the main chain).  That holds for both contractions: S = Q K^T and O = P V, with the probabilities P split the same way after
+// the fp32 online softmax in the exp2 domain.
+// Two passes.  (1) attention_split_kernel: k and v are split once per (image, head) into fp16 (hi, lo) pairs in a workspace.
+// (2) attention_tc5_kernel, flash-attention structure: nothing of size L x L touches HBM.  HBM traffic: q, k, v read once, the k / v
+// splits written once and read once (K/V tiles hit in L2 across the query tiles of a head), O written once.
+//
+// One CTA = 128 query rows of one (image, head) = the 128 lanes of tensor memory; thread t owns row t.  Keys stream in tiles of 64.
+// Per tile:  S = Q K^T   : 8 tcgen05.mma (M 128, K 16) from shared memory: Q_h [K_h; K_l] as one N = 128 MMA per k-step into TMEM
+//                          columns [0,64) main, [64,128) corr, then Q_l K_h onto corr
+//            softmax     : every thread reads its row of S with tcgen05.ld, p = exp2(s - m), writes P as fp16 (hi, lo) to shared memory
+//            O += P V    : 8 tcgen05.mma likewise (P_h [V_h | V_l], P_l V_h) into TMEM columns [128,192) main, [192,256) corr; O stays
+//                          in tensor memory over all key tiles and is rescaled there only when a row's maximum grows by more than 2^8
+// Operands sit in shared memory in the un-swizzled canonical core-matrix layouts (8 rows x 16 bytes = 128 contiguous bytes):
+// Q, K and P K-major; V MN-major, i.e. its row-major [key][dim] 16-byte pieces are only re-tiled, never transposed.
+// 256 TMEM columns and 112 KB of shared memory per CTA: two CTAs per SM, one's softmax under the other's MMAs.
+// Inside a CTA the tensor pipe runs ahead of the threads: S_{j+1} is issued as soon as every thread has read S_j (K tiles are
+// double-buffered), and O_{j-1} is waited for one tile late, so neither MMA group is waited for right after its issue.
+// K and V tiles are copied from the split workspace with cp.async as soon as the MMAs reading the buffer they replace have committed.
 #include <cuda_fp16.h>
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
 namespace pnp {
 
 constexpr int kAttD = 64;          // head dimension (ViT-L/16: 1024 / 16)
-constexpr int kAttTile = 64;       // keys per shared-memory tile = query rows per CTA
-constexpr int kAttPitch = 72;      // halves per shared row: 144 B, 16-byte aligned, conflict-free for ldmatrix and quad LDS.32
-
-__device__ __forceinline__ void mma_16816(float (&c)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
-    asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
-__device__ __forceinline__ void ldmatrix_x4(unsigned &r0, unsigned &r1, unsigned &r2, unsigned &r3, const __half *row_ptr) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-                 : "r"((unsigned)__cvta_generic_to_shared(row_ptr)));
-}
-
-__device__ __forceinline__ void ldmatrix_x4_trans(unsigned &r0, unsigned &r1, unsigned &r2, unsigned &r3, const __half *row_ptr) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
-                 : "r"((unsigned)__cvta_generic_to_shared(row_ptr)));
-}
-
-__device__ __forceinline__ void ldmatrix_x2_trans(unsigned &r0, unsigned &r1, const __half *row_ptr) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x2.trans.shared.b16 {%0,%1}, [%2];"
-                 : "=r"(r0), "=r"(r1)
-                 : "r"((unsigned)__cvta_generic_to_shared(row_ptr)));
-}
+constexpr int kAttTile = 64;       // keys per tile of the main kernel: the workspace rows are padded to a multiple of it
 
 // (x0, x1) -> packed half2 of the hi parts and of the 2^11-scaled lo parts (packed cvt.rn.f16x2.f32 conversions)
 __device__ __forceinline__ void split2(float x0, float x1, unsigned &hi, unsigned &lo) {
@@ -56,9 +41,9 @@ __device__ __forceinline__ void split2(float x0, float x1, unsigned &hi, unsigne
     lo = *reinterpret_cast<const unsigned *>(&ll);
 }
 
-// ---- pass 1: fp32 q, k, v -> fp16 (hi, lo) pairs, [3, 2, B, H, Lp, 64] with Lp = L rounded up to the tile (rows past L zero).
-// q is pre-multiplied by softmax_scale * log2(e) (the softmax runs on exp2), k and v by in_scale (a power of two: exact).
-// Done once per (image, head) instead of once per query tile inside the main kernel (7 query tiles share every K/V tile).
+// ---- pass 1: fp32 k, v -> fp16 (hi, lo) pairs, four [B, H, Lp, 64] planes k_hi, k_lo, v_hi, v_lo with Lp = L rounded up to the
+// tile (rows past L zero).  k and v are multiplied by in_scale (a power of two: exact); q is split by the main kernel.
+// Done once per (image, head) instead of once per query tile inside the main kernel (4 query tiles share every K/V tile at L = 442).
 __global__ void __launch_bounds__(256) attention_split_kernel(const float *__restrict__ qkv, __half *__restrict__ ws, int L, int Lp, int H,
                                                               int B, float in_scale, int *__restrict__ flag) {
     // grid = (Lp, B): one CTA per token row; its k and v parts are 2 x H x 64 contiguous floats of qkv.  No per-item divisions.
@@ -67,10 +52,10 @@ __global__ void __launch_bounds__(256) attention_split_kernel(const float *__res
     const int per_which = H * (kAttD / 4);                           // float4 pieces of the k (or v) part of one row
     bool bad = false;
     for (int i = threadIdx.x; i < 2 * per_which; i += blockDim.x) {
-        const int which = 1 + (i >= per_which), j = i - (which - 1) * per_which;   // 1 k, 2 v (q is split by the main kernel)
+        const int which = i >= per_which, j = i - which * per_which;   // 0 k, 1 v
         const int h = j >> 4, c4 = (j & 15) * 4;
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (l < L) v = ldg_stream4(qkv + (((size_t)b * L + l) * 3 + which) * H * kAttD + 4 * j);
+        if (l < L) v = ldg_stream4(qkv + (((size_t)b * L + l) * 3 + 1 + which) * H * kAttD + 4 * j);
         v.x *= in_scale; v.y *= in_scale; v.z *= in_scale; v.w *= in_scale;
         bad = bad || !(fabsf(v.x) <= 65504.f && fabsf(v.y) <= 65504.f && fabsf(v.z) <= 65504.f && fabsf(v.w) <= 65504.f);
         unsigned h01, l01, h23, l23;
@@ -83,243 +68,423 @@ __global__ void __launch_bounds__(256) attention_split_kernel(const float *__res
     if (bad && flag) *flag = 1;
 }
 
-__device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src));
+namespace tc5 {
+
+constexpr int BM = 128;            // query rows per CTA = TMEM lanes
+constexpr int BN = 64;             // keys per tile
+constexpr int D = 64;              // head dimension
+constexpr int NS = 256;            // softmax threads: two per query row
+constexpr int NT = NS + 32;        // + the warp whose lane 0 issues every tcgen05.mma
+constexpr int HC = 32;             // columns (keys of S, dims of O) per thread
+constexpr uint32_t LBO = 128;      // bytes between core matrices along K (adjacent)
+constexpr uint32_t SBO = 1024;     // bytes between 8-row groups along M/N (8 K-chunks of a 64-wide tile)
+constexpr uint32_t OFF_QH = 0, OFF_QL = 16384, OFF_K = 32768 /* 2 stages x (hi 8 KB, lo 8 KB) */, OFF_VH = 65536, OFF_VL = 73728,
+                   OFF_PH = 81920, OFF_PL = 98304, OFF_BAR = 114688, OFF_XCH = OFF_BAR + 64, SMEM_BYTES = OFF_XCH + 512;
+static_assert(2 * (SMEM_BYTES + 1024) <= 233472, "two CTAs per SM");
+constexpr uint32_t TM_S_MAIN = 0, TM_S_CORR = 64, TM_O_MAIN = 128, TM_O_CORR = 192, TM_COLS = 256;
+
+__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+// shared-memory matrix descriptor, no swizzle: start >> 4 | LBO >> 4 at 16 | SBO >> 4 at 32 | version 1 at 46
+__device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
+    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(LBO >> 4) << 16) | ((uint64_t)(SBO >> 4) << 32) | (1ull << 46);
+}
+// instruction descriptor, kind::f16: D fp32 (bit 4), A/B fp16, A K-major, B major at bit 16, N >> 3 at 17, M >> 4 at 24
+constexpr uint32_t kIdescS = (1u << 4) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+constexpr uint32_t kIdescS2 = (1u << 4) | ((uint32_t)(2 * BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);             // N = 128: hi and lo stacked
+constexpr uint32_t kIdescO2 = (1u << 4) | (1u << 16) | ((uint32_t)(2 * D >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+static_assert(TM_S_CORR == TM_S_MAIN + BN && TM_O_CORR == TM_O_MAIN + D && OFF_VL == OFF_VH + 8192, "stacked-N MMAs need adjacent halves");
+constexpr uint32_t kIdescO = (1u << 4) | (1u << 16) | ((uint32_t)(D >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+
+__device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
+    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d),
+                 "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
+                 : "memory");
+}
+__device__ __forceinline__ void umma_commit(uint32_t bar) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+    uint32_t done = 0;
+    for (int spin = 0; spin < (1 << 26); ++spin) {
+        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
+                     : "=r"(done)
+                     : "r"(bar), "r"(parity)
+                     : "memory");
+        if (done) return;
+    }
+    __trap();   // an MMA group that never commits is a bug: fail the launch instead of hanging the GPU
+}
+__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+    asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}\n" ::"r"(bar) : "memory");
+}
+__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+
+// 16 consecutive fp32 columns of this thread's TMEM lane
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
+    uint32_t r[16];
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
+                   "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                 : "r"(taddr)
+                 : "memory");
+#pragma unroll
+    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
+}
+
+__device__ __forceinline__ float ex2_approx(float x) {
+    float y;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+__device__ __forceinline__ void st_shared8(uint32_t addr, unsigned a, unsigned b) {
+    asm volatile("st.shared.v2.b32 [%0], {%1,%2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
+}
+
+__device__ __forceinline__ void cp_async16(uint32_t smem_dst, const void *gmem_src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gmem_src) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+__device__ __forceinline__ void cp_async_wait0() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
-// ---- pass 2: one CTA = 64 query rows of one (image, head); K/V tiles stream through a double-buffered cp.async pipeline.
-// out [B, L, H*64] fp32.
-// out [B, L, H*64] fp32 and / or out3 = its fp16 [h*hi_scale | l | h] operand split ([B*L, 3*H*64], see tf32x3.cu) for the
-// projection GEMM that follows.
-template <bool KX4, bool VX4>
-__global__ void __launch_bounds__(128, 2) attention_fp16x3_kernel(const float *__restrict__ qkv, const __half *__restrict__ ws,
-                                                                  float *__restrict__ out, __half *__restrict__ out3, int L, int Lp,
-                                                                  int H, int B, float q_scale, float hi_scale, int *__restrict__ flag) {
-    extern __shared__ __align__(16) __half att_smem[];   // [2 stages][kh, kl, vh, vl][64][72]
-    constexpr int kArr = kAttTile * kAttPitch;
-    const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * kAttTile;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int g = lane >> 2, tig = lane & 3;
-    const size_t plane = (size_t)B * H * Lp * kAttD;
-    const size_t head = ((size_t)b * H + h) * Lp * kAttD;
-    const __half *src[4] = {ws + 2 * plane + head, ws + 3 * plane + head, ws + 4 * plane + head, ws + 5 * plane + head};
+__device__ __forceinline__ void st_shared16(uint32_t addr, unsigned a, unsigned b, unsigned c, unsigned d) {
+    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
 
-    auto load_tile = [&](int stage, int k0) {   // 4 arrays x 64 rows x 128 B = 2048 16-byte pieces, 16 per thread
+// 16 consecutive 32-bit columns of this thread's TMEM lane, store
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const float (&v)[16]) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%16], {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15};" ::"r"(__float_as_uint(v[0])),
+                 "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])), "r"(__float_as_uint(v[4])),
+                 "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7])), "r"(__float_as_uint(v[8])),
+                 "r"(__float_as_uint(v[9])), "r"(__float_as_uint(v[10])), "r"(__float_as_uint(v[11])), "r"(__float_as_uint(v[12])),
+                 "r"(__float_as_uint(v[13])), "r"(__float_as_uint(v[14])), "r"(__float_as_uint(v[15])), "r"(taddr)
+                 : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
+constexpr float kRescaleThreshold = 8.0f;   // O and l are rescaled only when a row's maximum has grown by more than 2^8 (exp2 domain)
+
+// ws: the workspace of attention_split_kernel, [4][B,H,Lp,64] fp16 planes (k_hi, k_lo, v_hi, v_lo), Lp a multiple of 64.
+// 288 threads.  Warps 0-7 (softmax): thread t works on query row t & 127 (TMEM lane) and on the column half t >> 7 of S (keys) and
+// of O (dims); the two threads of a row exchange their partial row maximum through shared memory once per tile and their row sums
+// once at the end; they also copy the K / V tiles (cp.async).  Warp 8: lane 0 issues every tcgen05.mma (an issue blocks for ~100
+// cycles per MMA -- measured, profiles/experiments/probe_umma_timing.cu -- so it must not sit in a softmax thread's instruction stream).
+// O accumulates in tensor memory over all key tiles (the MMAs of tile j add to it).  The softmax subtracts a reference m_used that is
+// refreshed -- and O, l rescaled through tcgen05.ld / tcgen05.st -- only when the row maximum has outgrown it by more than 2^8: p stays
+// below 256, which fp16 (hi, lo) pairs hold as exactly as values below 1, and the result is the same softmax (any common shift is).
+// Hand-offs are mbarriers only: s_full / o_full (tcgen05.commit: an MMA group has finished), s_free (all 256 softmax threads have
+// read S_j), p_full (all 256 have written their part of P_j, finished any rescale of O and seen their copies land).
+__global__ void __launch_bounds__(NT, 2) attention_tc5_kernel(const float *__restrict__ qkv, const __half *__restrict__ ws,
+                                                              float *__restrict__ out, __half *__restrict__ out3, int L, int Lp, int H, int B,
+                                                              float q_scale, float hi_scale, int *__restrict__ flag) {
+    extern __shared__ __align__(1024) unsigned char smem[];
+    const uint32_t sbase = smem_u32(smem);
+    const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+    const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * BM;
+    const uint32_t bar_s = sbase + OFF_BAR, bar_o = sbase + OFF_BAR + 8, bar_s_free = sbase + OFF_BAR + 16, bar_p_full = sbase + OFF_BAR + 24;
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(smem + OFF_BAR + 32);
+    const int n_tiles = Lp / BN;
+
+    if (t == 0) {
+        mbar_init(bar_s, 1);
+        mbar_init(bar_o, 1);
+        mbar_init(bar_s_free, NS);
+        mbar_init(bar_p_full, NS);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == NS / 32) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TM_COLS) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+
+    if (warp == NS / 32) {
+        // ================================================================ MMA warp: lane 0 issues, the others wait at the end
+        tc_fence_before();
+        __syncthreads();                 // Q, K_0, K_1, V_0 are staged, TMEM is allocated, the barriers are initialised
+        tc_fence_after();
+        const uint32_t tmem = *tmem_slot;
+        if (lane == 0) {
+            // descriptors of the first k-step of every operand; k-step s is 256 bytes further: + 16 in the start-address field
+            const uint64_t d_qh = make_desc(sbase + OFF_QH), d_ql = make_desc(sbase + OFF_QL), d_ph = make_desc(sbase + OFF_PH),
+                           d_pl = make_desc(sbase + OFF_PL), d_vh = make_desc(sbase + OFF_VH), d_k0 = make_desc(sbase + OFF_K);
+            auto issue_s = [&](int tile) {   // S = Q K_tile^T : main = Qh Kh, corr = Ql Kh + Qh Kl
+                const uint64_t d_kh = d_k0 + (uint64_t)((tile & 1) * (16384 >> 4));
+                // B = [Kh ; Kl] stacked along N (the lo stage follows the hi stage: 8 more 8-row groups at the same SBO): one N = 128
+                // MMA per k-step gives Qh Kh in columns [0,64) and Qh Kl in [64,128); Ql Kh is added to the second half.  An MMA
+                // costs ~100 cycles for N = 64 and N = 128 alike: 8 MMAs, not 12.
 #pragma unroll
-        for (int a = 0; a < 4; ++a) {
-            __half *dst = att_smem + (stage * 4 + a) * kArr;
-            const __half *s = src[a] + (size_t)k0 * kAttD;
+                for (int s = 0; s < D / 16; ++s) umma(tmem + TM_S_MAIN, d_qh + 16 * s, d_kh + 16 * s, kIdescS2, s > 0);
 #pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const int idx = threadIdx.x + 128 * i;
-                const int row = idx >> 3, c8 = (idx & 7) * 8;
-                cp_async16(dst + row * kAttPitch + c8, s + row * kAttD + c8);
+                for (int s = 0; s < D / 16; ++s) umma(tmem + TM_S_CORR, d_ql + 16 * s, d_kh + 16 * s, kIdescS, 1);
+                umma_commit(bar_s);
+            };
+            issue_s(0);
+            for (int j = 0; j < n_tiles; ++j) {
+                const uint32_t par = (uint32_t)(j & 1);
+                if (j + 1 < n_tiles) {       // S_{j+1} once all 256 have read S_j (K_{j+1} landed before they arrived at p_full(j-1))
+                    mbar_wait(bar_s_free, par);
+                    tc_fence_after();
+                    issue_s(j + 1);
+                }
+                mbar_wait(bar_p_full, par);  // P_j and V_j are in shared memory, O has been rescaled where it had to be
+                tc_fence_after();
+#pragma unroll
+                for (int s2 = 0; s2 < BN / 16; ++s2) umma(tmem + TM_O_MAIN, d_ph + 16 * s2, d_vh + 16 * s2, kIdescO2, (j | s2) > 0);   // B = [Vh | Vl]
+#pragma unroll
+                for (int s2 = 0; s2 < BN / 16; ++s2) umma(tmem + TM_O_CORR, d_pl + 16 * s2, d_vh + 16 * s2, kIdescO, 1);
+                umma_commit(bar_o);
             }
+        }
+        __syncwarp();
+        tc_fence_before();
+        __syncthreads();                 // the softmax warps have read the final O (which also means: every MMA has completed)
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TM_COLS) : "memory");
+        return;
+    }
+
+    // ==================================================================== softmax warps
+    const int row = t & (BM - 1), hh = t >> 7;            // TMEM lane / column half
+    // [256] partial row maxima, rounded up to bf16: both threads of a row must subtract the SAME bound, and any bound >= the
+    // maximum is exact for a softmax; 16 bits keep two CTAs per SM inside the 228 KB
+    unsigned short *xch = reinterpret_cast<unsigned short *>(smem + OFF_XCH);
+    float *xch_l = reinterpret_cast<float *>(smem + OFF_K);   // [256] row sums (after the last S group the K stages are free)
+
+    // ---- K / V tile copies: 512 16-byte pieces per array, 2 per thread; piece (key, c = dim / 8)
+    const size_t plane = (size_t)B * H * Lp * D;
+    const __half *head = ws + ((size_t)b * H + h) * Lp * D;
+    auto load_k = [&](int tile) {   // into stage tile & 1
+        const uint32_t stage = sbase + OFF_K + (uint32_t)(tile & 1) * 16384;
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+            const int idx = t + NS * i, key = idx >> 3, c = idx & 7;
+            const uint32_t dst = (uint32_t)(key >> 3) * SBO + (uint32_t)c * LBO + (uint32_t)(key & 7) * 16;   // K-major: rows = keys
+            const __half *src = head + (size_t)(tile * BN + key) * D + c * 8;
+            cp_async16(stage + dst, src);
+            cp_async16(stage + 8192 + dst, src + plane);
+        }
+    };
+    auto load_v = [&](int tile) {
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+            const int idx = t + NS * i, key = idx >> 3, c = idx & 7;
+            const uint32_t dst = (uint32_t)c * SBO + (uint32_t)(key >> 3) * LBO + (uint32_t)(key & 7) * 16;   // MN-major: 8 dims contiguous
+            const __half *src = head + 2 * plane + (size_t)(tile * BN + key) * D + c * 8;   // planes v_hi, v_lo
+            cp_async16(sbase + OFF_VH + dst, src);
+            cp_async16(sbase + OFF_VL + dst, src + plane);
+        }
+    };
+    load_k(0);
+    if (n_tiles > 1) load_k(1);
+    load_v(0);
+    cp_async_commit();
+
+    // ---- the CTA's 128 query rows, pre-multiplied by in_scale * softmax_scale * log2(e), as K-major (hi, lo) rows; 16 threads read
+    // one row's 256 bytes (coalesced); all eight loads of a thread are in flight before the first conversion
+    {
+        const float *qb = qkv + (size_t)b * L * (size_t)(3 * H * D) + (size_t)h * D;
+        float4 a[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int idx = t + NS * i, r = idx >> 4, f = idx & 15;
+            a[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (q0 + r < L) a[i] = __ldg(reinterpret_cast<const float4 *>(qb + (size_t)(q0 + r) * (size_t)(3 * H * D) + 4 * f));
+        }
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int idx = t + NS * i, r = idx >> 4, f = idx & 15;
+            unsigned h0, h1, l0, l1;
+            split2(a[i].x * q_scale, a[i].y * q_scale, h0, l0);
+            split2(a[i].z * q_scale, a[i].w * q_scale, h1, l1);
+            const uint32_t off = (uint32_t)(r >> 3) * SBO + (uint32_t)(f >> 1) * LBO + (uint32_t)(r & 7) * 16 + (uint32_t)(f & 1) * 8;
+            st_shared8(sbase + OFF_QH + off, h0, h1);
+            st_shared8(sbase + OFF_QL + off, l0, l1);
+        }
+    }
+    cp_async_wait0();
+    fence_async_smem();
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = *tmem_slot;
+    const uint32_t lane_addr = tmem + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(hh * HC);
+
+    float m_used = -INFINITY, l = 0.f;
+    const uint32_t p_row = (uint32_t)(row >> 3) * SBO + (uint32_t)(row & 7) * 16 + (uint32_t)(hh * (HC / 8)) * LBO;
+
+    for (int j = 0; j < n_tiles; ++j) {
+        const int k0 = j * BN + hh * HC;     // first key of this thread's half of the tile
+        // ---- S_j is ready (issued one tile ago); its K stage is free for tile j + 2
+        mbar_wait(bar_s, (uint32_t)(j & 1));
+        tc_fence_after();
+        if (j + 2 < n_tiles) load_k(j + 2);
+        float s[HC];
+        {
+            float a0[16], c0[16], a1[16], c1[16];
+            tmem_ld16(lane_addr + TM_S_MAIN, a0);
+            tmem_ld16(lane_addr + TM_S_CORR, c0);
+            tmem_ld16(lane_addr + TM_S_MAIN + 16, a1);
+            tmem_ld16(lane_addr + TM_S_CORR + 16, c1);
+            tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+                s[i] = fmaf(c0[i], 1.0f / 2048.0f, a0[i]);
+                s[16 + i] = fmaf(c1[i], 1.0f / 2048.0f, a1[i]);
+            }
+        }
+        if (k0 + HC > L) {   // only the last tile holds keys past L
+#pragma unroll
+            for (int i = 0; i < HC; ++i)
+                if (k0 + i >= L) s[i] = -INFINITY;
+        }
+        float mx = s[0];
+#pragma unroll
+        for (int i = 1; i < HC; ++i) mx = fmaxf(mx, s[i]);
+        {
+            const unsigned u = __float_as_uint(mx);
+            const unsigned up = (u & 0x80000000u) ? (u & 0xFFFF0000u) : ((u + 0xFFFFu) & 0xFFFF0000u);   // towards +inf
+            mx = __uint_as_float(up);
+            xch[t] = (unsigned short)(up >> 16);
+        }
+        // the two warps that share these 32 rows meet at a named barrier (ids 1..4, 64 threads) and read each other's bound
+        asm volatile("bar.sync %0, 64;" ::"r"(1 + (warp & 3)) : "memory");
+        mx = fmaxf(mx, __uint_as_float((unsigned)xch[t ^ BM] << 16));
+        // ---- this thread is done with S_j (and with its partner's xch slot: the slot is rewritten only after S_{j+1} has been
+        // committed, which needs this arrival).  The tensor pipe starts on S_{j+1} once all 256 have arrived.
+        tc_fence_before();
+        mbar_arrive(bar_s_free);
+
+        // ---- P V_{j-1} has committed: the P and V buffers are free, and O may be rescaled
+        if (j > 0) {
+            mbar_wait(bar_o, (uint32_t)((j - 1) & 1));
+            tc_fence_after();
+            load_v(j);
         }
         cp_async_commit();
-    };
-    load_tile(0, 0);
-
-    // ---- this warp's 16 query rows as A fragments (hi and lo), pre-multiplied by in_scale * softmax_scale * log2(e)
-    const int r0 = q0 + warp * 16 + g, r1 = r0 + 8;
-    const size_t row_stride = (size_t)3 * H * kAttD;
-    const float *qb = qkv + (size_t)b * L * row_stride + (size_t)h * kAttD;
-    unsigned qh[4][4], ql[4][4];
+        // a row whose maximum has outgrown its reference by more than 2^8 gets a new reference; O (in TMEM) and l follow.  Both
+        // threads of a row see the same mx and take the same decision for their column halves; the branch is uniform per warp
+        // because tcgen05.ld / st are warp-wide.  Tile 0 only sets the reference (O is still empty).
+        const bool grow = mx > m_used + kRescaleThreshold;   // also true on tile 0 (m_used = -inf)
+        if (j > 0 && __any_sync(0xffffffffu, grow)) {
+            const float alpha = grow ? ex2_approx(m_used - mx) : 1.0f;
 #pragma unroll
-    for (int ks = 0; ks < 4; ++ks) {
-        const int c = 16 * ks + 2 * tig;
-        float2 v00 = make_float2(0.f, 0.f), v10 = v00, v01 = v00, v11 = v00;
-        if (r0 < L) {
-            v00 = *reinterpret_cast<const float2 *>(qb + (size_t)r0 * row_stride + c);
-            v01 = *reinterpret_cast<const float2 *>(qb + (size_t)r0 * row_stride + c + 8);
-        }
-        if (r1 < L) {
-            v10 = *reinterpret_cast<const float2 *>(qb + (size_t)r1 * row_stride + c);
-            v11 = *reinterpret_cast<const float2 *>(qb + (size_t)r1 * row_stride + c + 8);
-        }
-        split2(v00.x * q_scale, v00.y * q_scale, qh[ks][0], ql[ks][0]);
-        split2(v10.x * q_scale, v10.y * q_scale, qh[ks][1], ql[ks][1]);
-        split2(v01.x * q_scale, v01.y * q_scale, qh[ks][2], ql[ks][2]);
-        split2(v11.x * q_scale, v11.y * q_scale, qh[ks][3], ql[ks][3]);
-    }
-    float o_main[8][4], o_corr[8][4];
+            for (int c0 = 0; c0 < HC; c0 += 16) {
+                float a[16], cr[16];
+                tmem_ld16(lane_addr + TM_O_MAIN + c0, a);
+                tmem_ld16(lane_addr + TM_O_CORR + c0, cr);
+                tmem_ld_wait();
 #pragma unroll
-    for (int nt = 0; nt < 8; ++nt)
-#pragma unroll
-        for (int i = 0; i < 4; ++i) o_main[nt][i] = o_corr[nt][i] = 0.f;
-    float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-
-    const int n_tiles = Lp / kAttTile;
-    for (int t = 0; t < n_tiles; ++t) {
-        const int k0 = t * kAttTile, stage = t & 1;
-        if (t + 1 < n_tiles) {
-            load_tile(stage ^ 1, k0 + kAttTile);   // the buffer read two iterations ago: its readers passed the barrier below
-            cp_async_wait<1>();
-        } else {
-            cp_async_wait<0>();
-        }
-        __syncthreads();
-        const __half *s_kh = att_smem + (stage * 4 + 0) * kArr, *s_kl = att_smem + (stage * 4 + 1) * kArr;
-        const __half *s_vh = att_smem + (stage * 4 + 2) * kArr, *s_vl = att_smem + (stage * 4 + 3) * kArr;
-
-        // ---- S = Q K^T for 16 rows x 64 keys: main and correction accumulators; consecutive mma hit different accumulators
-        float s_main[8][4], s_corr[8][4];
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt)
-#pragma unroll
-            for (int i = 0; i < 4; ++i) s_main[nt][i] = s_corr[nt][i] = 0.f;
-        if (KX4) {
-            // B fragments of K^T through ldmatrix.x4 over the row-major [key][dim] tile: matrices (keys 8nt.., dims 16ks..+7),
-            // (same keys, dims +8) = b0, b1 of k-step ks, then the same pair for k-step ks+1; lane l supplies row (l & 7) of matrix l >> 3
-#pragma unroll
-            for (int kp = 0; kp < 2; ++kp) {           // k-steps 2kp, 2kp+1
-#pragma unroll
-                for (int nt = 0; nt < 8; ++nt) {
-                    const int off = (8 * nt + (lane & 7)) * kAttPitch + 32 * kp + 8 * (lane >> 3);
-                    unsigned h0, h1, h2, h3, l0_, l1_, l2_, l3_;
-                    ldmatrix_x4(h0, h1, h2, h3, s_kh + off);
-                    ldmatrix_x4(l0_, l1_, l2_, l3_, s_kl + off);
-                    mma_16816(s_main[nt], qh[2 * kp], h0, h1);
-                    mma_16816(s_corr[nt], ql[2 * kp], h0, h1);
-                    mma_16816(s_corr[nt], qh[2 * kp], l0_, l1_);
-                    mma_16816(s_main[nt], qh[2 * kp + 1], h2, h3);
-                    mma_16816(s_corr[nt], ql[2 * kp + 1], h2, h3);
-                    mma_16816(s_corr[nt], qh[2 * kp + 1], l2_, l3_);
-                }
+                for (int i = 0; i < 16; ++i) { a[i] *= alpha; cr[i] *= alpha; }
+                tmem_st16(lane_addr + TM_O_MAIN + c0, a);
+                tmem_st16(lane_addr + TM_O_CORR + c0, cr);
             }
-        } else {
-#pragma unroll
-            for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-                for (int nt = 0; nt < 8; ++nt) {
-                    const __half *krow_h = s_kh + (8 * nt + g) * kAttPitch + 2 * tig + 16 * ks;
-                    const __half *krow_l = s_kl + (8 * nt + g) * kAttPitch + 2 * tig + 16 * ks;
-                    const unsigned bh0 = *reinterpret_cast<const unsigned *>(krow_h), bh1 = *reinterpret_cast<const unsigned *>(krow_h + 8);
-                    const unsigned bl0 = *reinterpret_cast<const unsigned *>(krow_l), bl1 = *reinterpret_cast<const unsigned *>(krow_l + 8);
-                    mma_16816(s_main[nt], qh[ks], bh0, bh1);
-                    mma_16816(s_corr[nt], ql[ks], bh0, bh1);
-                    mma_16816(s_corr[nt], qh[ks], bl0, bl1);
-                }
-            }
+            tmem_st_wait();
+            l *= alpha;
         }
-        // ---- online softmax in the exp2 domain (fp32)
-        float mx0 = -INFINITY, mx1 = -INFINITY;
-        const bool tail = k0 + kAttTile > L;   // only the last tile holds keys past L (uniform branch)
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) s_main[nt][i] = fmaf(s_corr[nt][i], 1.0f / 2048.0f, s_main[nt][i]);
-            if (tail) {
-                const int key = k0 + 8 * nt + 2 * tig;
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    if (key + (i & 1) >= L) s_main[nt][i] = -INFINITY;
-            }
-            mx0 = fmaxf(mx0, fmaxf(s_main[nt][0], s_main[nt][1]));
-            mx1 = fmaxf(mx1, fmaxf(s_main[nt][2], s_main[nt][3]));
-        }
-        mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-        mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-        mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-        mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-        const float mn0 = fmaxf(m0, mx0), mn1 = fmaxf(m1, mx1);     // finite: every tile holds at least one key < L
-        const float a0 = exp2f(m0 - mn0), a1 = exp2f(m1 - mn1);
-        m0 = mn0; m1 = mn1;
-        float sum0 = 0.f, sum1 = 0.f;
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt) {
-            s_main[nt][0] = exp2f(s_main[nt][0] - mn0);
-            s_main[nt][1] = exp2f(s_main[nt][1] - mn0);
-            s_main[nt][2] = exp2f(s_main[nt][2] - mn1);
-            s_main[nt][3] = exp2f(s_main[nt][3] - mn1);
-            sum0 += s_main[nt][0] + s_main[nt][1];
-            sum1 += s_main[nt][2] + s_main[nt][3];
-            o_main[nt][0] *= a0; o_main[nt][1] *= a0; o_main[nt][2] *= a1; o_main[nt][3] *= a1;
-            o_corr[nt][0] *= a0; o_corr[nt][1] *= a0; o_corr[nt][2] *= a1; o_corr[nt][3] *= a1;
-        }
-        l0 = l0 * a0 + sum0;   // per-thread partial sums; reduced over the quad at the end
-        l1 = l1 * a1 + sum1;
+        if (grow) m_used = mx;
 
-        // ---- O += P V : P (this thread's C fragments) becomes the A fragments of the next mma, split into hi / lo
+        // ---- p = exp2(s - m_used) as fp16 (hi, lo) pairs, K-major rows of P
+        float sum = 0.f;
 #pragma unroll
-        for (int ks = 0; ks < 4; ++ks) {   // keys 16 ks .. 16 ks + 15
+        for (int c = 0; c < HC / 8; ++c) {
             unsigned ph[4], pl[4];
-            split2(s_main[2 * ks][0], s_main[2 * ks][1], ph[0], pl[0]);
-            split2(s_main[2 * ks][2], s_main[2 * ks][3], ph[1], pl[1]);
-            split2(s_main[2 * ks + 1][0], s_main[2 * ks + 1][1], ph[2], pl[2]);
-            split2(s_main[2 * ks + 1][2], s_main[2 * ks + 1][3], ph[3], pl[3]);
-            // B fragments of V[keys 16ks.., dims 8nt..]: ldmatrix.trans over the row-major [key][dim] tile; lanes 0-15 give the rows
-            if (VX4) {
-                // x4.trans: lanes 0-15 give the 16 key rows at dims 8nt.. (b0, b1 of n-tile nt), lanes 16-31 the same rows at dims
-                // 8(nt+1).. (b0, b1 of n-tile nt+1)
-                const int voff = (16 * ks + (lane & 15)) * kAttPitch + 8 * (lane >> 4);
 #pragma unroll
-                for (int nt = 0; nt < 8; nt += 2) {
-                    unsigned vh0, vh1, vh2, vh3, vl0, vl1, vl2, vl3;
-                    ldmatrix_x4_trans(vh0, vh1, vh2, vh3, s_vh + voff + 8 * nt);
-                    ldmatrix_x4_trans(vl0, vl1, vl2, vl3, s_vl + voff + 8 * nt);
-                    mma_16816(o_main[nt], ph, vh0, vh1);
-                    mma_16816(o_corr[nt], pl, vh0, vh1);
-                    mma_16816(o_corr[nt], ph, vl0, vl1);
-                    mma_16816(o_main[nt + 1], ph, vh2, vh3);
-                    mma_16816(o_corr[nt + 1], pl, vh2, vh3);
-                    mma_16816(o_corr[nt + 1], ph, vl2, vl3);
-                }
-            } else {
-                const int vrow = 16 * ks + (lane & 15);
-#pragma unroll
-                for (int nt = 0; nt < 8; ++nt) {
-                    unsigned vh0, vh1, vl0, vl1;
-                    ldmatrix_x2_trans(vh0, vh1, s_vh + vrow * kAttPitch + 8 * nt);
-                    ldmatrix_x2_trans(vl0, vl1, s_vl + vrow * kAttPitch + 8 * nt);
-                    mma_16816(o_main[nt], ph, vh0, vh1);
-                    mma_16816(o_corr[nt], pl, vh0, vh1);
-                    mma_16816(o_corr[nt], ph, vl0, vl1);
-                }
+            for (int i = 0; i < 4; ++i) {
+                const float p0 = ex2_approx(s[8 * c + 2 * i] - m_used), p1 = ex2_approx(s[8 * c + 2 * i + 1] - m_used);
+                sum += p0 + p1;
+                split2(p0, p1, ph[i], pl[i]);
             }
+            st_shared16(sbase + OFF_PH + p_row + c * LBO, ph[0], ph[1], ph[2], ph[3]);
+            st_shared16(sbase + OFF_PL + p_row + c * LBO, pl[0], pl[1], pl[2], pl[3]);
         }
-        __syncthreads();   // everyone is done with this stage before the next iteration's prefetch overwrites the other one's successor
+        l += sum;
+
+        // ---- P V_j may be issued once all 256 are here
+        cp_async_wait0();          // this thread's pieces of V_j (and K_{j+2}) have landed
+        fence_async_smem();
+        tc_fence_before();
+        mbar_arrive(bar_p_full);
     }
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-    const float inv0 = 1.0f / l0, inv1 = 1.0f / l1;
-    const int Dm = H * kAttD;
+    mbar_wait(bar_o, (uint32_t)((n_tiles - 1) & 1));
+    tc_fence_after();
+    float o[HC];
+#pragma unroll
+    for (int c0 = 0; c0 < HC; c0 += 16) {
+        float a[16], cr[16];
+        tmem_ld16(lane_addr + TM_O_MAIN + c0, a);
+        tmem_ld16(lane_addr + TM_O_CORR + c0, cr);
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 16; ++i) o[c0 + i] = fmaf(cr[i], 1.0f / 2048.0f, a[i]);
+    }
+    xch_l[t] = l;
+    tc_fence_before();
+    __syncthreads();
+
+    // ---- normalise; the rows go through shared memory (the V and P buffers are free) so that the global stores are whole
+    // 256-byte (fp32) / 128-byte (fp16) row segments.  16-byte pieces are XOR-swizzled by the row: conflict-free both ways.
+    const float inv = 1.0f / (l + xch_l[t ^ BM]);
+    const int Dm = H * D;
     bool bad = false;
 #pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-        const int c = h * kAttD + 8 * nt + 2 * tig;
+    for (int i = 0; i < HC; ++i) o[i] *= inv;
+    const uint32_t stage = sbase + OFF_VH;
+    if (out) {
 #pragma unroll
-        for (int half_row = 0; half_row < 2; ++half_row) {
-            const int r = half_row ? r1 : r0;
-            if (r >= L) continue;
-            const float inv = half_row ? inv1 : inv0;
-            const float x0 = fmaf(o_corr[nt][2 * half_row], 1.0f / 2048.0f, o_main[nt][2 * half_row]) * inv;
-            const float x1 = fmaf(o_corr[nt][2 * half_row + 1], 1.0f / 2048.0f, o_main[nt][2 * half_row + 1]) * inv;
-            const size_t m = (size_t)b * L + r;
-            if (out) *reinterpret_cast<float2 *>(out + m * Dm + c) = make_float2(x0, x1);
-            if (out3) {   // [h * hi_scale | l | h] of the attention output, ready for the projection GEMM
-                unsigned hh, ll;
-                split2(x0, x1, hh, ll);
-                __half2 hs = __hmul2(*reinterpret_cast<__half2 *>(&hh), __float2half2_rn(hi_scale));   // a power of two: exact
+        for (int c = 0; c < HC / 4; ++c) {   // fp32 [128][16 pieces]
+            const int piece = hh * (HC / 4) + c;
+            st_shared16(stage + (uint32_t)row * 256 + (uint32_t)((piece ^ (row & 7)) * 16), __float_as_uint(o[4 * c]), __float_as_uint(o[4 * c + 1]),
+                        __float_as_uint(o[4 * c + 2]), __float_as_uint(o[4 * c + 3]));
+        }
+        asm volatile("bar.sync 5, %0;" ::"n"(NS) : "memory");
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int idx = t + NS * i, r = idx >> 4, piece = idx & 15;
+            if (q0 + r < L) {
+                const uint4 v = *reinterpret_cast<const uint4 *>(smem + OFF_VH + r * 256 + ((piece ^ (r & 7)) * 16));
+                *reinterpret_cast<uint4 *>(out + ((size_t)b * L + q0 + r) * Dm + (size_t)h * D + 4 * piece) = v;
+            }
+        }
+        if (out3) asm volatile("bar.sync 5, %0;" ::"n"(NS) : "memory");
+    }
+    if (out3) {   // [h * hi_scale | l | h] of the attention output, ready for the projection GEMM: three fp16 [128][8 pieces] arrays
+        const __half2 hs2 = __float2half2_rn(hi_scale);
+#pragma unroll
+        for (int c = 0; c < HC / 8; ++c) {
+            unsigned hv[4], lv[4], sc[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const float x0 = o[8 * c + 2 * k], x1 = o[8 * c + 2 * k + 1];
+                split2(x0, x1, hv[k], lv[k]);
+                const __half2 hsv = __hmul2(*reinterpret_cast<__half2 *>(&hv[k]), hs2);   // a power of two: exact
+                sc[k] = *reinterpret_cast<const unsigned *>(&hsv);
                 bad = bad || !(fabsf(x0 * hi_scale) <= 65504.f && fabsf(x1 * hi_scale) <= 65504.f);
-                __half *row = out3 + m * 3 * Dm;
-                *reinterpret_cast<unsigned *>(row + c) = *reinterpret_cast<unsigned *>(&hs);
-                *reinterpret_cast<unsigned *>(row + Dm + c) = ll;
-                *reinterpret_cast<unsigned *>(row + 2 * Dm + c) = hh;
+            }
+            const int piece = hh * (HC / 8) + c;
+            const uint32_t off = (uint32_t)row * 128 + (uint32_t)((piece ^ (row & 7)) * 16);
+            st_shared16(stage + off, sc[0], sc[1], sc[2], sc[3]);
+            st_shared16(stage + 16384 + off, lv[0], lv[1], lv[2], lv[3]);
+            st_shared16(stage + 32768 + off, hv[0], hv[1], hv[2], hv[3]);
+        }
+        asm volatile("bar.sync 5, %0;" ::"n"(NS) : "memory");
+#pragma unroll
+        for (int i = 0; i < 12; ++i) {
+            const int idx = t + NS * i, arr = idx >> 10, r = (idx >> 3) & (BM - 1), piece = idx & 7;
+            if (q0 + r < L) {
+                const uint4 v = *reinterpret_cast<const uint4 *>(smem + OFF_VH + arr * 16384 + r * 128 + ((piece ^ (r & 7)) * 16));
+                *reinterpret_cast<uint4 *>(out3 + ((size_t)b * L + q0 + r) * 3 * Dm + (size_t)arr * Dm + (size_t)h * D + 8 * piece) = v;
             }
         }
     }
     if (bad && flag) *flag = 1;
 }
 
-// attention_tc5.cu: the same contraction on tcgen05.mma / tensor memory (the default main kernel)
-int launch_attention_tc5(const float *qkv, const __half *ws, float *out, __half *out3, int L, int Lp, int H, int B, float q_scale,
-                         float hi_scale, int *flag, cudaStream_t st);
+}  // namespace tc5
 
 }  // namespace pnp
 
@@ -328,7 +493,7 @@ using namespace pnp;
 extern "C" size_t pnp_attention_fp16x3_workspace_bytes(int B, int L, int H, int D) {
     if (B < 0 || L < 1 || H < 1 || D != kAttD) return 0;
     const size_t Lp = (size_t)ceil_div(L, kAttTile) * kAttTile;
-    return 6 * (size_t)B * H * Lp * kAttD * sizeof(__half);   // (planes 2..5 = k_hi, k_lo, v_hi, v_lo are used)
+    return 4 * (size_t)B * H * Lp * kAttD * sizeof(__half);   // k_hi, k_lo, v_hi, v_lo
 }
 
 extern "C" int pnp_attention_fp16x3(const float *qkv, float in_scale, float softmax_scale, float *out, uint16_t *out3, float out3_hi_scale,
@@ -342,39 +507,15 @@ extern "C" int pnp_attention_fp16x3(const float *qkv, float in_scale, float soft
     if (B == 0) return PNP_OK;
     cudaStream_t st = as_stream(stream);
     const int Lp = ceil_div(L, kAttTile) * kAttTile;
-    const size_t smem = 2 * 4 * (size_t)kAttTile * kAttPitch * sizeof(__half);   // 73 728 B: two CTAs per SM
-    // fragment loads: bit 0 = K through ldmatrix.x4 (else quad LDS.32), bit 1 = V through ldmatrix.x4.trans (else x2.trans).  All four
-    // run within 1.5 % of each other (0.353-0.359 ms per call at 35 x 16 x 442, profiles/experiments/r2_attention_variants.py): the
-    // kernel is bound by the mma pipe and its latency at 2 CTAs per SM, not by fragment loads.  Default 2 (229 registers).
-    static const int variant = getenv("PNP_ATT_VARIANT") ? atoi(getenv("PNP_ATT_VARIANT")) : 2;
+    const cudaError_t e = allow_smem(tc5::attention_tc5_kernel, tc5::SMEM_BYTES);
+    if (e != cudaSuccess) return cuda_err(e);
     __half *ws = reinterpret_cast<__half *>(workspace);
     const bool timed = prof::on(kAttention, st);
     if (timed) prof::begin(kAttention, st);
     attention_split_kernel<<<dim3(Lp, B), 256, 0, st>>>(qkv, ws, L, Lp, H, B, in_scale, overflow_flag);
-    const dim3 grid_main(Lp / kAttTile, H, B);
     const float q_scale = in_scale * softmax_scale * 1.4426950408889634f;
-    __half *o3 = reinterpret_cast<__half *>(out3);
-    // main kernel: tcgen05.mma with TMEM accumulators (attention_tc5.cu) unless PNP_ATT_TCGEN05=0 asks for the mma.sync one below
-    const char *env_tc5 = getenv("PNP_ATT_TCGEN05");   // read per call: tests compare the two kernels in one process
-    const int use_tc5 = env_tc5 ? atoi(env_tc5) : 1;
-    if (use_tc5) {
-        const int rc = launch_attention_tc5(qkv, ws, out, o3, L, Lp, H, B, q_scale, out3_hi_scale, overflow_flag, st);
-        if (timed) prof::end(kAttention, st);
-        return rc;
-    }
-#define PNP_ATT(KX, VX)                                                                                                       \
-    do {                                                                                                                      \
-        cudaError_t e = allow_smem(attention_fp16x3_kernel<KX, VX>, smem); \
-        if (e != cudaSuccess) return cuda_err(e);                                                                             \
-        attention_fp16x3_kernel<KX, VX><<<grid_main, 128, smem, st>>>(qkv, ws, out, o3, L, Lp, H, B, q_scale, out3_hi_scale, overflow_flag); \
-    } while (0)
-    switch (variant & 3) {
-        case 1: PNP_ATT(true, false); break;
-        case 2: PNP_ATT(false, true); break;
-        case 3: PNP_ATT(true, true); break;
-        default: PNP_ATT(false, false); break;
-    }
-#undef PNP_ATT
+    tc5::attention_tc5_kernel<<<dim3(ceil_div(L, tc5::BM), H, B), tc5::NT, tc5::SMEM_BYTES, st>>>(
+        qkv, ws, out, reinterpret_cast<__half *>(out3), L, Lp, H, B, q_scale, out3_hi_scale, overflow_flag);
     if (timed) prof::end(kAttention, st);
     return launch_status();
 }

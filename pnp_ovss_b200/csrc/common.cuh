@@ -71,7 +71,8 @@ __device__ __forceinline__ float warp_sum(float v) {
 }
 
 // ---- order-preserving float <-> uint32 keys for atomicMin/atomicMax; NaN is sticky ----
-// max side: +NaN maps to the largest key; min side: NaN is canonicalised to the smallest key.
+// A NaN is stored as the largest key on the max side and as the smallest on the min side:
+// key 0xffffffff decodes to u = 0x7fffffff (NaN); key 0 decodes to u = 0xffffffff (NaN): both stay NaN.
 __device__ __forceinline__ unsigned f2key(float f) {
     unsigned u = __float_as_uint(f);
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -80,9 +81,6 @@ __device__ __forceinline__ float key2f(unsigned k) {
     unsigned u = (k & 0x80000000u) ? (k & 0x7fffffffu) : ~k;
     return __uint_as_float(u);
 }
-__device__ __forceinline__ unsigned f2key_max(float f) { return (f != f) ? 0xffffffffu : f2key(f); }  // NaN -> top
-__device__ __forceinline__ unsigned f2key_min(float f) { return (f != f) ? 0u : f2key(f); }           // NaN -> bottom
-// key 0xffffffff decodes to u = 0x7fffffff (NaN); key 0 decodes to u = 0xffffffff (NaN): both stay NaN.
 
 // min/max that propagate NaN like torch.min/max and numpy
 __device__ __forceinline__ float nan_min(float a, float b) { return (a != a || b != b) ? __int_as_float(0x7fc00000) : fminf(a, b); }

@@ -14,8 +14,6 @@
 // and uses FMA / __expf (its inputs already carry expf ulps); the marginals stay within 1e-3 of the restatement (tests).
 #include <math.h>
 
-#include <stdlib.h>
-
 #include <algorithm>
 #include <type_traits>
 
@@ -91,28 +89,6 @@ __global__ void __launch_bounds__(256) splat_kernel(LatticeView L, const float *
             acc = f4_add(acc, f4_mul(xv, __ldg(L.csr_w + k)));
         }
         *reinterpret_cast<float4 *>(vb + (size_t)(v + 1) * L.vp + 4 * ch) = acc;
-    }
-}
-
-// Experiment (PNP_SPLAT_ATOMIC=1, bilateral lattice only): the transposed formulation -- one thread per (pixel, chunk) reads its
-// Q row once (coalesced) and adds w * norm * Q into its d+1 vertex rows with vector float atomics (red.global.add.v4.f32).
-// No CSR, perfectly balanced warps, but the summation order -- hence the low bits of every marginal -- changes from run to
-// run, so it is NOT the default: results of the measurement in profiles/README.md.
-__global__ void __launch_bounds__(256) splat_atomic_kernel(LatticeView L, const float *__restrict__ x, float *__restrict__ values, int Cp,
-                                                           long long n_lp) {
-    const int nch = Cp >> 2;
-    const long long total = n_lp * nch;
-    for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
-        const long long lp = idx / nch;
-        const int ch = (int)(idx - lp * nch);
-        float4 q = ldg_stream4(x + lp * Cp + 4 * ch);
-        const float nr = __ldg(L.norm + lp);
-        q = f4_mul(q, nr);
-        for (int j = 0; j < L.Dp1; ++j) {
-            const int o = __ldg(L.offset + lp * L.Dp1 + j) + 1;
-            const float w = __ldg(L.bary + lp * L.Dp1 + j);
-            atomicAdd(reinterpret_cast<float4 *>(values + (size_t)o * L.vp + 4 * ch), f4_mul(q, w));
-        }
     }
 }
 
@@ -667,56 +643,30 @@ __global__ void __launch_bounds__(kUnaryPix) unpack_nc_to_cn_kernel(const float 
 }
 
 // ------------------------------------------------------------------------------------------ host helpers
-// CTAs per SM of the grid-stride kernels.  Measured on B200 (profiles/sweep_grid.py): the lattice blur is fastest with
-// exactly one resident wave (8 CTAs x 148 SMs: every SM streams one contiguous slice, no tail), the splat with many
-// more CTAs than fit (its CSR rows differ in length, so late CTAs fill the holes), the mean-field update with 8.
-// PNP_GRID_MULT_{BLUR,SPLAT,UPDATE} override for tuning runs.
-static inline int env_mult(const char *name, int dflt) {
-    const char *e = getenv(name);
-    int v = e ? atoi(e) : dflt;
-    return v > 0 ? v : dflt;
-}
-static inline int mult_blur() { static int m = env_mult("PNP_GRID_MULT_BLUR", 8); return m; }
+// CTAs per SM of the grid-stride kernels.  Measured on B200: the lattice blur is fastest with exactly one resident wave
+// (8 CTAs x 148 SMs: every SM streams one contiguous slice, no tail), the splat with many more CTAs than fit (its CSR rows
+// differ in length, so late CTAs fill the holes), the mean-field update with 8.
+constexpr int kMultBlur = 8;
 // Splat: the wider the rows, the more CTAs.  Measured per CRF pass (10 launches, profiles/time_other_configs.py; grid = 148 SMs x mult
 // CTAs of 256 threads, grid-stride): 21 channels  64: 4.69 ms, 512: 5.26;  59 channels  128: 9.2, 256: 9.3, 512: 9.9;
 // 81 channels @448  64: 24.5, 128: 21.3, 256: 19.6, 512: 20.0;  150 channels  64: 24.0, 128: 21.0, 256: 19.6, 512: 19.3, 1024: 20.4,
 // one chunk per CTA (4096): 23.2.  (ncu at 150 channels, mult 64: 8.6 GB of DRAM reads per launch for 2.4 GB of Q, L2 hit rate 30 %:
 // every CTA of a long grid-stride loop hops through the whole batch.  Handing chunks of consecutive vertices out in order from a
 // global counter to one resident wave was also measured: 21.7 ms at 150 channels -- better than mult 64, worse than mult 256.)
-static inline int mult_splat(int nch) {
-    static int forced = env_mult("PNP_GRID_MULT_SPLAT", 1 << 30);
-    if (forced != (1 << 30)) return forced;
-    return nch <= 8 ? 64 : (nch <= 16 ? 128 : 256);
-}
+static inline int mult_splat(int nch) { return nch <= 8 ? 64 : (nch <= 16 ? 128 : 256); }
 // Update: one resident wave for narrow rows; with wide rows more, shorter-lived CTAs hide the gather latency a little better
 // (per CRF pass, mult 8 / 16 / 32 / 64: 21 channels 5.36 / 5.36 / 5.42 / 5.48 ms, 81 channels @448 29.2 / 28.1 / 27.0 / 27.3, 150
 // channels 31.2 / 30.3 / 29.2 / 28.8).
-static inline int mult_update(int nch) {
-    static int forced = env_mult("PNP_GRID_MULT_UPDATE", 1 << 30);
-    if (forced != (1 << 30)) return forced;
-    return nch <= 8 ? 8 : 32;
-}
+static inline int mult_update(int nch) { return nch <= 8 ? 8 : 32; }
 static inline int grid_for(long long work_items, int threads, int mult = 16) {
     return (int)std::max<long long>(1, std::min<long long>((work_items + threads - 1) / threads, (long long)kNumSMs * mult));
 }
 
-// Row pitch of the vertex-value buffers.  Default: rows packed at Cp floats.  PNP_VALUE_PITCH=1 pads rows so that none
-// straddles a 128-byte line (96-byte rows cross a boundary every other row); measured on B200 it does not pay: the
-// gather kernels do not speed up and the HBM-bound lattice blur slows by 9 % (profiles/README.md), so it stays off.
-static inline int value_pitch(int Cp) {
-    static const int padded = env_mult("PNP_VALUE_PITCH", 2) == 1;
-    if (!padded) return Cp;
-    const int bytes = Cp * 4;
-    if (bytes <= 128) {
-        int p = 16;
-        while (p < bytes) p <<= 1;
-        return p / 4;
-    }
-    return (bytes + 127) / 128 * 32;
-}
+// Vertex-value rows are packed at Cp floats (vp = Cp).  Padding rows so that none straddles a 128-byte line was measured on
+// B200 and does not pay: the gather kernels do not speed up and the HBM-bound lattice blur slows by 9 % (profiles/README.md).
 static inline LatticeView view_for(const pnp_lattice *lat, int Cp) {
     LatticeView L = make_view(lat);
-    L.vp = value_pitch(Cp);
+    L.vp = Cp;
     return L;
 }
 
@@ -733,33 +683,18 @@ static const float *run_splat_blur(const LatticeView &L, const float *x, float *
     const int gy = L.shared ? B : 1;
     const int div = L.shared ? std::min(B, 8) : 1;
     const int gx_splat = std::max(1, grid_for((long long)(L.M + 1) * nch, 256, mult_splat(nch)) / div);
-    const int gx = std::max(1, grid_for((long long)(L.M + 1) * nch, 256, mult_blur()) / div);
+    const int gx = std::max(1, grid_for((long long)(L.M + 1) * nch, 256, kMultBlur) / div);
     const int id_splat = L.shared ? kSplatSpatial : kSplatBilateral;
     const int id_blur = L.shared ? kBlurAxisSpatial : kBlurAxisBilateral;
-    static const int atomic_splat = env_mult("PNP_SPLAT_ATOMIC", 2) == 1;
-    if (atomic_splat && !L.shared && normalized) {   // experiment: pixel-order vector-atomic splat (non-deterministic sums)
-        const bool timed = prof::on(id_splat, st);
-        if (timed) prof::begin(id_splat, st);
-        cudaMemsetAsync(va, 0, (size_t)(L.M + 1) * L.vp * sizeof(float), st);
-        const long long n_lp = (long long)B * L.N;
-        splat_atomic_kernel<<<grid_for(n_lp * nch, 256, 16), 256, 0, st>>>(L, x, va, Cp, n_lp);
-        if (timed) prof::end(id_splat, st);
-    } else {
-        PNP_LAUNCH(id_splat, st, splat_kernel<<<dim3(gx_splat, gy), 256, 0, st>>>(L, x, va, Cp, normalized));
-    }
+    PNP_LAUNCH(id_splat, st, splat_kernel<<<dim3(gx_splat, gy), 256, 0, st>>>(L, x, va, Cp, normalized));
     float *src = va, *dst = vb;
     // Two axes per launch halve the HBM traffic of the blur but re-gather the first axis at both neighbours; measured on
     // B200 that pays up to ~340-byte rows (21 ch: 0.187 vs 0.232 ms, 81 ch @448: 23.6 vs 27.5 ms per pass) and loses with
     // 600-byte rows (150 ch: 44.4 vs 38.6 ms), where one launch per axis already runs at the HBM roofline.
-    static const int fuse_mode = env_mult("PNP_BLUR_FUSE", 1);        // 2: never fuse (tuning)
-    static const int fuse_max_cp = env_mult("PNP_BLUR_FUSE_MAX_CP", 112);
-    const bool fuse_pairs = fuse_mode != 2 && Cp <= fuse_max_cp;
-    static const int mult2 = env_mult("PNP_GRID_MULT_BLUR2", 8);
-    const int gx2 = std::max(1, grid_for((long long)(L.M + 1) * nch, 256, mult2) / div);
     int j = 0;
-    if (fuse_pairs) {
+    if (Cp <= 112) {
         for (; j + 1 < L.Dp1; j += 2) {  // axes (0,1), (2,3), (4,5): two passes per launch
-            PNP_LAUNCH(id_blur, st, blur_axis2_kernel<<<dim3(gx2, gy), 256, 0, st>>>(L, src, dst, j, j + 1, Cp));
+            PNP_LAUNCH(id_blur, st, blur_axis2_kernel<<<dim3(gx, gy), 256, 0, st>>>(L, src, dst, j, j + 1, Cp));
             std::swap(src, dst);
         }
     }
@@ -843,18 +778,15 @@ extern "C" int pnp_crf_inference(const pnp_lattice *const *lattices, const float
     int LPP = 0, CPL = 0;
     {
         double best_eff = 0.0;
-        static const int forced_cpl = env_mult("PNP_UPDATE_CPL", 9);  // tuning: force chunks per lane (1..4)
         for (int cpl = 1; cpl <= 6; ++cpl) {
             if (cpl == 5) continue;
-            if (forced_cpl <= 6 && cpl != forced_cpl) continue;
             int lpp = (nch_all + cpl - 1) / cpl;
             if (lpp > 32) continue;
             double eff = (double)(32 / lpp) * nch_all / (32.0 * cpl);
             if (eff >= best_eff - 1e-9) { best_eff = eff; LPP = lpp; CPL = cpl; }  // ties: more chunks per lane wins (measured)
         }
     }
-    static const int occ3_min_nch = env_mult("PNP_UPDATE_OCC3_MIN_NCH", 12);   // rows of >= 192 bytes
-    const bool occ3 = (CPL == 4 || CPL == 6) && nch_all >= occ3_min_nch;
+    const bool occ3 = (CPL == 4 || CPL == 6) && nch_all >= 12;   // rows of >= 192 bytes
     const bool warp_path = CPL > 0 && Wimg > 0 && (long long)Himg * Wimg == N && (long long)B * N < (1ll << 31) / Cp;
     const int grid_w = (int)std::max<long long>(
         1, std::min<long long>((long long)B * ((Himg + kTile - 1) / kTile) * ((Wimg + kTile - 1) / kTile), (long long)kNumSMs * mult_update(nch_all)));

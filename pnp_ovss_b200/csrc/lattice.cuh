@@ -19,7 +19,7 @@ struct LatticeView {
     int shared;              // 1: one image's lattice applied to every image
     int N;                   // pixels per image
     float alpha;             // 1 / (1 + 2^-d)
-    int vp;                  // floats between consecutive rows of a vertex-value buffer (>= Cp; set per call)
+    int vp;                  // floats between consecutive rows of a vertex-value buffer (= Cp; set per call by view_for)
 };
 
 static inline LatticeView make_view(const pnp_lattice *lat) {

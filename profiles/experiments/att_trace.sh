@@ -4,7 +4,7 @@
 set -e
 cd "$(dirname "$0")/../../pnp_ovss_b200/csrc"
 mkdir -p build_trace
-for f in lib tf32x3 attention attention_tc5 xattn gradcam upsample_blur lattice crf confusion; do
+for f in lib tf32x3 attention xattn gradcam upsample_blur lattice crf confusion; do
   /usr/local/cuda/bin/nvcc -O3 -std=c++17 -lineinfo -gencode arch=compute_100a,code=sm_100a -Xcompiler -fPIC --fmad=true -DPNP_ATT_TRACE -c $f.cu -o build_trace/$f.o &
 done
 wait

@@ -1,11 +1,10 @@
 """GradCAM distance from an fp64 autograd pass (4 images, full-size model, block 8 / head 9) and time per 35-image pass for:
 native fp32 as torch runs it by default (cuDNN may use TF32 for the patch-embedding convolution), strict fp32 (all TF32 off),
-3xTF32 with one depth-3K GEMM, 3xTF32 with the corrections in a second GEMM."""
+3xTF32 with the corrections in a second GEMM.  (The one-depth-3K-GEMM arm and its switch are at commit 5c46d18.)"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import torch
 import bench
-from pnp_ovss_b200 import blip_itm
 from pnp_ovss_b200.blip_itm import BlipITM
 
 dev = torch.device("cuda:0")
@@ -41,7 +40,4 @@ torch.backends.cudnn.allow_tf32 = False
 run("strict fp32 (cudnn.allow_tf32 = False)")
 torch.backends.cudnn.allow_tf32 = True
 model.gemm_precision = "3xtf32"
-blip_itm.MM3_SEPARATE_CORRECTION = False
-run("3xtf32, one depth-3K GEMM")
-blip_itm.MM3_SEPARATE_CORRECTION = True
 run("3xtf32, corrections in a second GEMM")

@@ -1,4 +1,4 @@
-"""CPU restatement of the arithmetic contract of the tcgen05 attention kernel (pnp_ovss_b200/csrc/attention_tc5.cu), in numpy:
+"""CPU restatement of the arithmetic contract of the tcgen05 attention kernel (pnp_ovss_b200/csrc/attention.cu), in numpy:
   * every fp32 operand x is split exactly into x = h + l 2^-11 (h = fp16(x), l = fp16((x - h) 2^11)) and a product a.b is evaluated as
     a_h b_h + 2^-11 (a_l b_h + a_h b_l) with fp32 accumulation (the dropped a_l b_l term is ~2^-22 relative);
   * keys stream in tiles of 64; a row's softmax subtracts a reference m_used that is refreshed -- and O, l rescaled -- only when the

@@ -85,6 +85,19 @@ def test_product_never_imports_the_oracle():
             assert "oracle" not in open(os.path.join(pkg, "csrc", fn)).read().replace("CPU oracle", "")
 
 
+def test_library_reads_no_environment():
+    """Every choice a kernel launch makes is fixed in the source or derived from its arguments: no environment switch, so
+    concurrent calls from several host threads cannot see different configurations."""
+    csrc = os.path.join(ROOT, "pnp_ovss_b200", "csrc")
+    for fn in os.listdir(csrc):
+        if fn.endswith((".cu", ".cuh", ".h", ".cpp")):
+            assert "getenv" not in open(os.path.join(csrc, fn)).read(), fn
+    header = open(HEADER).read()
+    for name in ("PNP_ATT_TCGEN05", "PNP_ATT_VARIANT", "PNP_SPLAT_ATOMIC", "PNP_VALUE_PITCH", "PNP_GRID_MULT", "PNP_BLUR_FUSE",
+                 "PNP_UPDATE_CPL", "PNP_UPDATE_OCC3_MIN_NCH"):
+        assert name not in header, name
+
+
 def test_header_cites_reference_lines():
     text = open(HEADER).read()
     for cite in ("MED:267-283", "BITM:415-433", "DRV:810-853", "DRV:638-647", "DRV:1149-1153", "DRV:1030-1074", "DRV:1106-1112"):

@@ -618,27 +618,18 @@ def test_attention_fp16x3_is_fp32_grade(dev, ops, B, L, H):
 
 
 @pytest.mark.parametrize("B,L,H", [(1, 1, 1), (2, 64, 3), (1, 129, 2), (3, 442, 4), (1, 1000, 1)])
-def test_attention_tcgen05_matches_the_mma_sync_kernel(dev, ops, B, L, H, monkeypatch):
-    """The tcgen05 / tensor-memory kernel (default) and the mma.sync kernel (PNP_ATT_TCGEN05=0) evaluate the same split products
-    with the same fp32 softmax; they differ only in summation order (64-key tiles, hi/lo accumulators).  Both within fp32 grade of
-    an fp64 evaluation, within 4e-6 of each other, deterministic, and rows past L / keys past L never leak in (tile edges at 1, 64,
-    129, 1000)."""
+def test_attention_fp16x3_tile_edges(dev, ops, B, L, H):
+    """At the edges of the 64-key and 128-row tiles (L = 1, 64, 129, 1000): deterministic, within 4e-6 of an fp64 evaluation (rows
+    past L / keys past L never leak in), and the operand-split output is the split of the kernel's own fp32 output."""
     g = torch.Generator().manual_seed(17 * L + H)
     qkv = torch.randn(B, L, 3, H, 64, generator=g).to(dev)
     q, k, v = (qkv[:, :, i].permute(0, 2, 1, 3) for i in range(3))
     truth = torch.nn.functional.scaled_dot_product_attention(q.double(), k.double(), v.double()).permute(0, 2, 1, 3).reshape(B, L, H * 64)
-    monkeypatch.setenv("PNP_ATT_TCGEN05", "1")
-    new = ops.attention_fp16x3(qkv)
-    new2 = ops.attention_fp16x3(qkv)
-    monkeypatch.setenv("PNP_ATT_TCGEN05", "0")
-    old = ops.attention_fp16x3(qkv)
+    got = ops.attention_fp16x3(qkv)
+    got2 = ops.attention_fp16x3(qkv)
     sc = truth.abs().max().item()
-    assert torch.equal(new, new2)
-    assert (new.double() - truth).abs().max().item() / sc <= 4e-6
-    assert (old.double() - truth).abs().max().item() / sc <= 4e-6
-    assert (new - old).abs().max().item() / sc <= 4e-6
-    # the operand-split output of both kernels is the split of their own fp32 output
+    assert torch.equal(got, got2)
+    assert (got.double() - truth).abs().max().item() / sc <= 4e-6
     flag = torch.zeros(1, dtype=torch.int32, device=dev)
-    monkeypatch.setenv("PNP_ATT_TCGEN05", "1")
-    assert torch.equal(ops.attention_fp16x3(qkv, flag=flag, split_hi_scale=4.0), ops.fp16_split3(new, 1.0, 4.0, flag))
+    assert torch.equal(ops.attention_fp16x3(qkv, flag=flag, split_hi_scale=4.0), ops.fp16_split3(got, 1.0, 4.0, flag))
     assert int(flag.item()) == 0
