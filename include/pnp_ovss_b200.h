@@ -284,7 +284,12 @@ int pnp_layernorm_fp16_split3(const float *x, const float *residual, float resid
  * split of k and v. */
 size_t pnp_attention_fp16x3_workspace_bytes(int B, int L, int H, int D);
 /* out and / or out3 (at least one): out3 [B*L, 3*H*D] fp16 is the [h * out3_hi_scale | l | h] operand split of the output
- * (pnp_fp16_split3's layout), written straight from the accumulators for the projection GEMM that follows. */
+ * (pnp_fp16_split3's layout), written straight from the accumulators for the projection GEMM that follows.
+ * *overflow_flag (device int, optional) is set to 1, and never cleared, when the result may not be fp32-grade: a k or v value
+ * times in_scale, or a q value times in_scale * softmax_scale * log2(e), outside fp16's range (or NaN); a row whose scores reach
+ * 2^11 in magnitude in the exp2 domain (about 1420 in natural units, scores = q.k * softmax_scale), where the bf16 row bound the
+ * softmax subtracts is too coarse for the fp16 (hi, lo) pairs of the probabilities; or, with out3, an output times out3_hi_scale
+ * outside fp16's range.  Below that magnitude the result is fp32-grade whatever the spread of a row's scores. */
 int pnp_attention_fp16x3(const float *qkv, float in_scale, float softmax_scale, float *out, uint16_t *out3,
                          float out3_hi_scale, void *workspace, size_t workspace_bytes, int *overflow_flag, int B, int L,
                          int H, int D, pnp_stream_t stream);

@@ -286,6 +286,7 @@ __global__ void __launch_bounds__(NT, 2) attention_tc5_kernel(const float *__res
 
     // ---- the CTA's 128 query rows, pre-multiplied by in_scale * softmax_scale * log2(e), as K-major (hi, lo) rows; 16 threads read
     // one row's 256 bytes (coalesced); all eight loads of a thread are in flight before the first conversion
+    bool q_bad = false;   // a scaled q value outside fp16's range (or NaN): its hi part would be inf
     {
         const float *qb = qkv + (size_t)b * L * (size_t)(3 * H * D) + (size_t)h * D;
         float4 a[8];
@@ -298,9 +299,11 @@ __global__ void __launch_bounds__(NT, 2) attention_tc5_kernel(const float *__res
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
             const int idx = t + NS * i, r = idx >> 4, f = idx & 15;
+            const float x0 = a[i].x * q_scale, x1 = a[i].y * q_scale, x2 = a[i].z * q_scale, x3 = a[i].w * q_scale;
+            q_bad = q_bad || !(fabsf(x0) <= 65504.f && fabsf(x1) <= 65504.f && fabsf(x2) <= 65504.f && fabsf(x3) <= 65504.f);
             unsigned h0, h1, l0, l1;
-            split2(a[i].x * q_scale, a[i].y * q_scale, h0, l0);
-            split2(a[i].z * q_scale, a[i].w * q_scale, h1, l1);
+            split2(x0, x1, h0, l0);
+            split2(x2, x3, h1, l1);
             const uint32_t off = (uint32_t)(r >> 3) * SBO + (uint32_t)(f >> 1) * LBO + (uint32_t)(r & 7) * 16 + (uint32_t)(f & 1) * 8;
             st_shared8(sbase + OFF_QH + off, h0, h1);
             st_shared8(sbase + OFF_QL + off, l0, l1);
@@ -430,7 +433,11 @@ __global__ void __launch_bounds__(NT, 2) attention_tc5_kernel(const float *__res
     // 256-byte (fp32) / 128-byte (fp16) row segments.  16-byte pieces are XOR-swizzled by the row: conflict-free both ways.
     const float inv = 1.0f / (l + xch_l[t ^ BM]);
     const int Dm = H * D;
-    bool bad = false;
+    // The bound both threads of a row subtract is bf16, so it can sit one bf16 ulp above the row maximum: the largest p of the row is
+    // then as small as 2^-ulp.  For |m_used| < 2^11 the ulp is at most 8 and p_max >= 2^-8 stays in fp16's normal range; beyond it
+    // the (hi, lo) pairs of P lose bits or flush to zero.  m_used only grows; tiles taken under an earlier, coarser bound weigh at
+    // most 2^-8 after the rescale that replaced it (2^-2048 if it was below -4096), so the final bound is the one to test.
+    bool bad = q_bad || !(fabsf(m_used) < 2048.f);
 #pragma unroll
     for (int i = 0; i < HC; ++i) o[i] *= inv;
     const uint32_t stage = sbase + OFF_VH;
