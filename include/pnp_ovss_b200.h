@@ -58,6 +58,7 @@ int pnp_xattn_softmax_fwd(const float *scores, const float *key_mask, float *pro
 /* Backward of the above fused with the GradCAM product of BITM:415-433 for ONE head.
  *   dscores = probs * (dprobs - sum_k(probs*dprobs)) * scale                (autograd of MED:267-274)
  *   gradcam[b,t-1,p] = probs[b,head,t,p+1] * max(dprobs[b,head,t,p+1],0) * token_mask[b,t]   for t >= 1
+ *   (max(NaN,0) = NaN, like torch's clamp; the products are rounded left to right)
  * probs, dprobs, dscores [B,heads,T,K]; token_mask int64 [B,token_mask_stride] (the max_length=500 padded
  * attention_mask, BITM:415-416), token_mask_stride >= T; gradcam [B,T-1,K-1] (= [B,T-1,P,P]).
  * dscores == NULL: only the GradCAM of `head` is produced (frozen-weights mode, SURVEY 7.4).
@@ -88,7 +89,8 @@ int pnp_token_merge(const float *gradcam, const int32_t *seg_start, const int32_
  *   pred = gradcam[b] with the n_prev already-chosen cells zeroed            -> ensemble_r (optional)
  *   agg  = round == 0 ? pred + pred : agg + pred                              (optional)
  *   score[p] = sum_{t in [row_lo,row_hi)} gradcam[b,t,p] (sequential fp32), chosen cells := 0
- *   new = the save_len largest scores (ties: larger index ranks higher, = a stable ascending argsort's tail)
+ *   new = the save_len largest scores (ties: larger index ranks higher, = a stable ascending argsort's tail;
+ *         as in numpy, NaN ranks above +inf and -0 ties with +0)
  *   chosen[b, n_prev : n_prev+save_len] = new (ascending score order)
  *   imgs[b,:,16r:16r+16,16c:16c+16] = 0 and norm_imgs[b,16r:16r+16,16c:16c+16,:] = 0 for the new cells
  * gradcam, ensemble_r, agg [B,Tm,P*P]; chosen int32 [B,chosen_stride]; imgs [B,3,S,S] or NULL; norm_imgs

@@ -26,12 +26,20 @@ __global__ void __launch_bounds__(256) token_merge_kernel(const float *__restric
 
 constexpr int kMaxCells = 1024;  // P*P <= 1024 (P <= 32)
 
+// Order-preserving key of a DropOut score under numpy's sort order: -0 ties with +0, and every NaN ties with the
+// others above +inf (np.argsort puts NaN last).
+__device__ __forceinline__ unsigned int score_key(float s) {
+    if (s != s) return 0xFFFFFFFFu;
+    const unsigned int u = __float_as_uint(s == 0.f ? 0.f : s);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
 __global__ void __launch_bounds__(512) salience_dropout_round_kernel(const float *__restrict__ gradcam, float *__restrict__ ensemble_r,
                                                                      float *__restrict__ agg, int32_t *__restrict__ chosen,
                                                                      int chosen_stride, int n_prev, float *__restrict__ imgs,
                                                                      float *__restrict__ norm_imgs, int Tm, int P, int patch,
                                                                      int row_lo, int row_hi, int save_len, int round) {
-    __shared__ float s_score[kMaxCells];
+    __shared__ unsigned int s_key[kMaxCells];
     __shared__ unsigned char s_dropped[kMaxCells];
     __shared__ int s_new[32];
     const int b = blockIdx.x;
@@ -60,17 +68,19 @@ __global__ void __launch_bounds__(512) salience_dropout_round_kernel(const float
     for (int p = threadIdx.x; p < PP; p += blockDim.x) {
         float acc = 0.f;
         for (int t = row_lo; t < row_hi; ++t) acc = __fadd_rn(acc, g[(long long)t * PP + p]);
-        s_score[p] = s_dropped[p] ? 0.f : acc;
+        s_key[p] = score_key(s_dropped[p] ? 0.f : acc);
     }
     __syncthreads();
 
-    // DRV:643-647: argsort(score)[-save_len:] by rank counting (ties: larger index ranks higher)
+    // DRV:643-647: argsort(score, kind="stable")[-save_len:] by rank counting (ties: larger index ranks higher).
+    // (key, index) is a total order, so the ranks are a permutation of 0..PP-1 and every s_new slot is written
+    // exactly once, whatever the scores hold.
     for (int p = threadIdx.x; p < PP; p += blockDim.x) {
-        const float sp = s_score[p];
+        const unsigned int kp = s_key[p];
         int rank = 0;
         for (int q = 0; q < PP; ++q) {
-            float sq = s_score[q];
-            rank += (sq > sp) || (sq == sp && q > p);
+            const unsigned int kq = s_key[q];
+            rank += (kq > kp) || (kq == kp && q > p);
         }
         if (rank < save_len) s_new[save_len - 1 - rank] = p;
     }

@@ -91,8 +91,10 @@ __global__ void __launch_bounds__(256) softmax_bwd_gradcam_kernel(const float *_
                 dv[i] = dp[k];
                 if (kFull) inner = fmaf(pv[i], dv[i], inner);
                 if (cam_row && k >= 1) {
-                    // BITM:427: cams * grads.clamp(0) * mask   (left to right, separately rounded)
-                    g[k - 1] = __fmul_rn(__fmul_rn(pv[i], fmaxf(dv[i], 0.f)), m);
+                    // BITM:427: cams * grads.clamp(0) * mask   (left to right, separately rounded).  torch's clamp
+                    // keeps a NaN gradient NaN; fmaxf alone would turn it into 0.
+                    const float dc = dv[i] != dv[i] ? dv[i] : fmaxf(dv[i], 0.f);
+                    g[k - 1] = __fmul_rn(__fmul_rn(pv[i], dc), m);
                 }
             } else {
                 pv[i] = 0.f;

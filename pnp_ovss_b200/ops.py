@@ -61,6 +61,12 @@ def softmax_bwd_gradcam(probs, dprobs, token_mask, head, scale=0.125, need_dscor
             raise PnpError("token_mask must be [B, >=T]")
         stride = token_mask.shape[1]
         gradcam = torch.empty((B, T - 1, K - 1), dtype=torch.float32, device=probs.device)
+        if not 0 <= int(head) < h:
+            raise PnpError("head out of range")
+    if all(t is None or t.numel() == 0 for t in (dscores, gradcam)):
+        # nothing to write (B == 0, or frozen mode with T == 1): an empty tensor's null data pointer would read as "output not
+        # requested" to the library, which refuses a call that requests no output
+        return dscores, gradcam
     check(_lib.load().pnp_xattn_softmax_bwd_gradcam(_p(probs), _p(dprobs), _p(dscores), _p(token_mask if need_gradcam else None),
                                                     stride, _p(gradcam), B, h, T, K, float(scale), int(head), _stream()),
           "pnp_xattn_softmax_bwd_gradcam")
