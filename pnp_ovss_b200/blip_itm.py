@@ -14,6 +14,7 @@ Two ways to get GradCAM (both end in pnp_xattn_softmax_bwd_gradcam):
   * reference-style (`full_backward=True`): everything requires grad and loss.backward() runs through the whole
     model like BITM:399-404; the autograd.Function's backward emits dscores and the GradCAM in one pass."""
 import math
+import types
 
 import torch
 import torch.nn as nn
@@ -107,13 +108,14 @@ def _w16(weight, bias=None):
     return torch.cat(cols, 1).contiguous(), 2.0 ** (11 - b)
 
 
-def _mm16(x16, w16):
+def _mm16(x16, w16, out=None):
     """2^11 * (x W^T) at fp32-grade accuracy as ONE fp16 tensor-core GEMM (fp32 accumulate and output) over the tripled
     operands: x_h W_h 2^11 + x_l W_h + x_h W_l, with x = x_h + x_l 2^-11.  The caller takes the 2^11 back (a power of two)."""
-    return torch.mm(x16.reshape(-1, x16.shape[-1]), w16.t(), out_dtype=torch.float32).view(*x16.shape[:-1], w16.shape[0])
+    y = torch.mm(x16.reshape(-1, x16.shape[-1]), w16.t(), out_dtype=torch.float32, out=out)
+    return y.view(*x16.shape[:-1], w16.shape[0])
 
 
-def _mm3(x3, w3, bias=None):
+def _mm3(x3, w3, bias=None, out=None):
     """y = x W^T (+ bias) at fp32-grade accuracy on the TF32 tensor cores over the tripled operands (fp32 accumulate; the
     dropped x_lo W_lo term is ~2^-22 relative).  Still plain torch dense contractions (cuBLAS).
 
@@ -127,11 +129,40 @@ def _mm3(x3, w3, bias=None):
     try:
         K = w3.shape[1] // 3
         x2 = x3.reshape(-1, 3 * K)
-        y = F.linear(x2[:, :K], w3[:, :K], bias)
+        xh, wh = x2[:, :K], w3[:, :K].t()
+        y = torch.mm(xh, wh, out=out) if bias is None else torch.addmm(bias, xh, wh, out=out)   # = F.linear on 2-D operands
         y.addmm_(x2[:, K:], w3[:, K:].t())
         return y.view(*x3.shape[:-1], w3.shape[0])
     finally:
         torch.backends.cuda.matmul.allow_tf32 = prev
+
+
+# The two operand forms of the split GEMM modes.  `prep(W, b)` makes the right-hand operand (weight, hi_scale, b) of a frozen
+# weight; `split` / `ln` / `gelu` write the matching left-hand operand of an activation (the fp16 forms raise `flag` when a
+# value leaves fp16's range); `mm` multiplies the two, and the product carries the factor `scale`, which the next producer
+# takes back exactly (a power of two).
+#   3xtf32: [hi | lo | hi] fp32, two launches (_mm3), the bias added by the GEMM from the live parameter, scale 1.
+#   3xfp16: [h 2^a | l | h] fp16, one launch (_mm16), scale 2^11; a bias is folded into 8 more weight columns (_w16), and `ln`
+#           writes the matching [FP16_BIAS_ONE, 1, 0 x 6] columns for an operand that carries one.
+_FORMS = {
+    "3xtf32": types.SimpleNamespace(
+        scale=1.0,
+        prep=lambda w, b=None: (_w3(w), 1.0, b),
+        mm=lambda x3, op, out=None: _mm3(x3, op[0], op[2], out),
+        split=lambda x, in_scale, op, flag: ops.tf32_split3(x),
+        ln=lambda x, norm, op, flag, r=None, rb=None, **kw: ops.layernorm_tf32_split3(
+            x, norm.weight, norm.bias, norm.eps, residual=r, residual_bias=rb, **kw),
+        gelu=lambda x, bias, op, flag: ops.gelu_tf32_split3(x, bias)),
+    "3xfp16": types.SimpleNamespace(
+        scale=FP16_OUT_SCALE,
+        prep=lambda w, b=None: _w16(w, b) + (b,),
+        mm=lambda x16, op, out=None: _mm16(x16, op[0], out),
+        split=lambda x, in_scale, op, flag: ops.fp16_split3(x, in_scale, op[1], flag),
+        ln=lambda x, norm, op, flag, r=None, rb=None, **kw: ops.layernorm_fp16_split3(
+            x, norm.weight, norm.bias, norm.eps, residual=r, residual_scale=1.0 / FP16_OUT_SCALE, residual_bias=rb, hi_scale=op[1],
+            flag=flag, bias_one=None if op[2] is None else FP16_BIAS_ONE, **kw),
+        gelu=lambda x, bias, op, flag: ops.gelu_fp16_split3(x, bias, 1.0 / FP16_OUT_SCALE, op[1], flag)),
+}
 
 
 class _Linear3(torch.autograd.Function):
@@ -306,13 +337,11 @@ class BlipITM(nn.Module):
             nn.init.ones_(m.weight)
             nn.init.zeros_(m.bias)
 
-    _CACHES = ("_w3_cache", "_text3_cache", "_text_graphs", "_text_graph_stamp", "_vit_graphs", "_kv_buffers", "_fp16_flags")
-
     def __deepcopy__(self, memo):
-        """Copies the module without its derived state (weight splits, K/V buffers, captured CUDA graphs): all of it is rebuilt
-        on first use, and a CUDA graph cannot be copied."""
+        """Copies the module without its derived state (see _refresh; rebuilt on first use, and a CUDA graph cannot be copied)
+        and with clear fp16 overflow flags."""
         import copy
-        saved = {k: self.__dict__.pop(k) for k in self._CACHES if k in self.__dict__}
+        saved = {k: self.__dict__.pop(k) for k in ("_derived", "_fp16_flags") if k in self.__dict__}
         try:
             new = self.__class__.__new__(self.__class__)
             memo[id(self)] = new
@@ -329,12 +358,16 @@ class BlipITM(nn.Module):
         return _TextEncoderView(self)
 
     def load_lavis_checkpoint(self, path_or_state_dict):
-        """Weights of the reference's LAVIS BlipITM (YAML:10) -> this model; see lavis_compat.load_lavis_state_dict."""
+        """Weights of the reference's LAVIS BlipITM (YAML:10) -> this model, with clear fp16 overflow flags; see
+        lavis_compat.load_lavis_state_dict."""
         from .lavis_compat import load_lavis_state_dict
         sd = path_or_state_dict
         if not isinstance(sd, dict):
             sd = torch.load(sd, map_location="cpu")
-        return load_lavis_state_dict(self, sd)
+        ignored = load_lavis_state_dict(self, sd)
+        for flag in self.__dict__.get("_fp16_flags", {}).values():
+            flag.zero_()
+        return ignored
 
     # ---- pieces -----------------------------------------------------------------------------------
     def _tokenize(self, text_input, device):
@@ -356,57 +389,61 @@ class BlipITM(nn.Module):
     # ---- "3xtf32" / "3xfp16": the frozen-weight encoder pass with every large GEMM on the tensor cores at fp32-grade accuracy
     SPLIT_MODES = ("3xtf32", "3xfp16")
 
+    def _refresh(self):
+        """Everything derived from the parameters -- weight operands per split mode, text-side _Linear3 splits, the K/V output
+        buffers and the captured CUDA graphs, which hold the addresses of all of these -- lives in one dict that is dropped
+        when the stamp of the parameters changes.  The stamp is (data_ptr, _version) of every weight and bias: it sees in-place
+        edits (load_state_dict copies in place) and moves (.to()).  Called once per forward() / gradcam() of a split mode
+        (_encode).  -> True when no parameter requires grad (the split paths serve frozen weights only)."""
+        stamp, grad, mods = [], False, [self]
+        for m in mods:
+            mods.extend(m._modules.values())
+            for p in m._parameters.values():
+                stamp.append((p.data_ptr(), p._version))
+                grad = grad or p.requires_grad
+        if self.__dict__.get("_derived", {}).get("stamp") != stamp:
+            self.__dict__["_derived"] = {"stamp": stamp, "weights": {}, "text": {}, "kv": {}, "graphs": {}}
+        return not grad
+
+    def _cache(self, name):
+        """One part of the derived state of the current parameters (see _refresh)."""
+        if "_derived" not in self.__dict__:
+            self._refresh()
+        return self.__dict__["_derived"][name]
+
     def _weights3(self, mode="3xtf32"):
-        """Tripled splits of the frozen weights for `mode` ([W_hi | W_hi | W_lo] fp32, see _w3; or fp16 with its activation
-        scale, see _w16), rebuilt when a parameter changes."""
-        ve = self.visual_encoder
-        params = [ve.patch_embed.weight] + [p for blk in ve.blocks for p in (blk.qkv.weight, blk.proj.weight, blk.fc1.weight, blk.fc2.weight)]
-        params += [p for lyr in self.layer for p in (lyr.crossattention.self.key.weight, lyr.crossattention.self.value.weight)]
-        stamp = tuple((p.data_ptr(), p._version) for p in params)
-        caches = self.__dict__.setdefault("_w3_cache", {})
-        cache = caches.get(mode)
-        if cache is None or cache["stamp"] != stamp:
-            half = mode == "3xfp16"
-            prep = (lambda w, b=None: _w16(w, b)) if half else (lambda w, b=None: (_w3(w), 1.0))
+        """Operands of the frozen encoder weights in `mode`'s form (see _FORMS)."""
+        cache = self._cache("weights")
+        if mode not in cache:
+            prep = _FORMS[mode].prep
+            ve = self.visual_encoder
+            xs = [lyr.crossattention.self for lyr in self.layer]
             with torch.no_grad():
-                xs = [lyr.crossattention.self for lyr in self.layer]
-                kv_bias = torch.cat([b for x in xs for b in (x.key.bias, x.value.bias)], 0).contiguous()
-                cache = {
-                    "stamp": stamp,
+                cache[mode] = {
                     "patch": prep(ve.patch_embed.weight.reshape(ve.patch_embed.weight.shape[0], -1)),
-                    # (qkv with its bias folded into the operand in the fp16 form, proj, fc1, fc2)
                     "blocks": [(prep(blk.qkv.weight, blk.qkv.bias), prep(blk.proj.weight), prep(blk.fc1.weight), prep(blk.fc2.weight))
                                for blk in ve.blocks],
                     # key/value projections of all cross-attention blocks as one [layers*2*hidden, 3*enc_width (+8)] operand
-                    "kv": prep(torch.cat([w for x in xs for w in (x.key.weight, x.value.weight)], 0), kv_bias),
-                    "kv_bias": kv_bias,
+                    "kv": prep(torch.cat([w for x in xs for w in (x.key.weight, x.value.weight)], 0),
+                               torch.cat([b for x in xs for b in (x.key.bias, x.value.bias)], 0).contiguous()),
                 }
-            caches[mode] = cache
-        return cache
+        return cache[mode]
 
-    def _text_linear(self):
-        """lin(module, x) for the text side: in the tensor-core modes (frozen weights, CUDA) every nn.Linear of the BERT layers
-        runs through _Linear3 (forward and backward on the TF32 tensor cores at fp32 grade); plain module call otherwise."""
-        if self.gemm_precision not in self.SPLIT_MODES or any(p.requires_grad for p in self.layer.parameters()):
-            return _plain_linear
-        cache = self.__dict__.setdefault("_text3_cache", {})
-
-        def lin(module, x):
-            if not x.is_cuda or module.in_features % 4 or module.out_features % 4:
-                return module(x)
-            w = module.weight
-            ent = cache.get(id(module))
-            if ent is None or ent[0] != (w.data_ptr(), w._version):
-                with torch.no_grad():
-                    ent = ((w.data_ptr(), w._version), _w3(w), _w3(w.t().contiguous()))
-                cache[id(module)] = ent
-            return _Linear3.apply(x, ent[1], ent[2], module.bias)
-
-        return lin
+    def _linear3(self, module, x):
+        """lin(module, x) of the text side on the split path: an nn.Linear of the BERT layers through _Linear3 (forward and
+        backward on the TF32 tensor cores at fp32 grade)."""
+        if module.in_features % 4 or module.out_features % 4:
+            return module(x)
+        cache = self._cache("text")
+        if module not in cache:
+            with torch.no_grad():
+                cache[module] = (_w3(module.weight), _w3(module.weight.t().contiguous()))
+        return _Linear3.apply(x, *cache[module], module.bias)
 
     def fp16_overflow_flag(self, device):
         """Device int32 raised by the 3xFP16 operand kernels when an activation does not fit fp16; read it once per run
-        (`check_fp16_overflow`), not per pass."""
+        (`check_fp16_overflow`), not per pass.  Not part of the derived state (_refresh): captured graphs hold its address, and
+        an overflow seen before a weight change is still reported."""
         flags = self.__dict__.setdefault("_fp16_flags", {})
         key = str(device)
         if key not in flags:
@@ -421,135 +458,103 @@ class BlipITM(nn.Module):
     def _vit3(self, imgs, want_plain=False, mode="3xtf32"):
         """ViT-L forward (VIT:274-290) under no_grad with the GEMM operands prepared by the fused split kernels:
         residual add + LayerNorm + split, GELU + split, plain split.  Returns (enc3 [B,L,3D] split, enc [B,L,D] or None).
-        mode "3xfp16": the products carry a factor 2^11 that the next fused kernel takes back (inv)."""
+        Every product carries the factor of `mode`'s form (2^11 in 3xfp16), which the next fused kernel takes back (inv)."""
         ve = self.visual_encoder
-        w = self._weights3(mode)
-        half = mode == "3xfp16"
-        inv = 1.0 / FP16_OUT_SCALE if half else 1.0
-        flag = self.fp16_overflow_flag(imgs.device) if half else None
-        mm = _mm16 if half else _mm3
-
-        def split(x, in_scale, wt):
-            return ops.fp16_split3(x, in_scale, wt[1], flag) if half else ops.tf32_split3(x)
-
-        def ln(x, norm, wt, r=None, rb=None, fold_bias=False, **kw):
-            if half:
-                return ops.layernorm_fp16_split3(x, norm.weight, norm.bias, norm.eps, residual=r, residual_scale=inv, residual_bias=rb,
-                                                 hi_scale=wt[1], flag=flag, bias_one=FP16_BIAS_ONE if fold_bias else None, **kw)
-            return ops.layernorm_tf32_split3(x, norm.weight, norm.bias, norm.eps, residual=r, residual_bias=rb, **kw)
-
+        f, w = _FORMS[mode], self._weights3(mode)
+        inv = 1.0 / f.scale
+        flag = self.fp16_overflow_flag(imgs.device)
         B, _, S, _ = imgs.shape
         ps = ve.patch_embed.kernel_size[0]
         G = S // ps
         D = ve.pos_embed.shape[-1]
         patches = imgs.view(B, 3, G, ps, G, ps).permute(0, 2, 4, 1, 3, 5).reshape(B * G * G, 3 * ps * ps).contiguous()
-        pe = torch.add(ve.patch_embed.bias, mm(split(patches, 1.0, w["patch"]), w["patch"][0]), alpha=inv).view(B, G * G, D)
+        pe = torch.add(ve.patch_embed.bias, f.mm(f.split(patches, 1.0, w["patch"], flag), w["patch"]), alpha=inv).view(B, G * G, D)
         x = (torch.cat([ve.cls_token.expand(B, -1, -1), pe], 1) + ve.pos_embed).contiguous()
         L = x.shape[1]
         r = rb = None
         for blk, (w_qkv, w_proj, w_fc1, w_fc2) in zip(ve.blocks, w["blocks"]):
-            h3, _ = ln(x, blk.norm1, w_qkv, r, rb, fold_bias=True)
-            # fp16 form: the GEMM adds the bias itself (operand columns) and q, k, v come out times 2^11 -- a power of two that
-            # the attention's scale (2^-22 / sqrt(d)) and the next split (2^-11) take back exactly
-            qkv = mm(h3, w_qkv[0]) if half else _mm3(h3, w_qkv[0], blk.qkv.bias)
+            # q, k, v come out times the form's factor -- a power of two that the attention's scale and the next split take back
+            qkv = f.mm(f.ln(x, blk.norm1, w_qkv, flag, r, rb)[0], w_qkv)
             hd = D // blk.heads
-            if half and hd == 64:
+            if mode == "3xfp16" and hd == 64:
                 # the attention itself on the fp16 tensor cores with the same hi/lo split (pnp_attention_fp16x3): unscaled output
                 a3 = ops.attention_fp16x3(qkv.view(B, L, 3, blk.heads, hd), inv, 1.0 / math.sqrt(hd), flag, split_hi_scale=w_proj[1])
-                r = mm(a3, w_proj[0])
             else:
                 qkv = qkv.view(B, L, 3, blk.heads, hd).permute(2, 0, 3, 1, 4)
                 a = F.scaled_dot_product_attention(qkv[0], qkv[1], qkv[2], scale=inv * inv / math.sqrt(hd))
-                r = mm(split(a.transpose(1, 2).reshape(B, L, D).contiguous(), inv, w_proj), w_proj[0])
-            h3, _ = ln(x, blk.norm2, w_fc1, r, blk.proj.bias)
-            f = mm(h3, w_fc1[0])
-            g3 = (ops.gelu_fp16_split3(f, blk.fc1.bias, inv, w_fc2[1], flag) if half else ops.gelu_tf32_split3(f, blk.fc1.bias))
-            r, rb = mm(g3, w_fc2[0]), blk.fc2.bias
-        return ln(x, ve.norm, w["kv"], r, rb, fold_bias=True, split=True, plain=want_plain)
+                a3 = f.split(a.transpose(1, 2).reshape(B, L, D).contiguous(), inv, w_proj, flag)
+            r = f.mm(a3, w_proj)
+            h = f.mm(f.ln(x, blk.norm2, w_fc1, flag, r, blk.proj.bias)[0], w_fc1)
+            r, rb = f.mm(f.gelu(h, blk.fc1.bias, w_fc2, flag), w_fc2), blk.fc2.bias
+        return f.ln(x, ve.norm, w["kv"], flag, r, rb, split=True, plain=want_plain)
 
     def _cross_kv3(self, enc3, mode="3xtf32"):
         """key(enc) / value(enc) of every cross-attention block (MED:201-221) in one GEMM -> list of (k, v, s) with k, v
         [B,L,hidden] carrying the factor s (2^11 in the fp16 form: the cross-attention takes it back, see CrossAttentionSelf)."""
-        w = self._weights3(mode)
+        f, kv = _FORMS[mode], self._weights3(mode)["kv"]
         n = len(self.layer)
-        half = mode == "3xfp16"
         # One persistent output buffer per shape: the text-pass CUDA graph reads K/V at fixed addresses, so the GEMM writes there
         # directly and nothing is copied.  (Passes on one stream are ordered; a pass never outlives the next one's GEMM.)
-        bufs = self.__dict__.setdefault("_kv_buffers", {})
-        M, N = enc3.shape[0] * enc3.shape[1], w["kv"][0].shape[0]
+        bufs = self._cache("kv")
+        M, N = enc3.shape[0] * enc3.shape[1], kv[0].shape[0]
         key = (M, N, str(enc3.device))
         if key not in bufs:
             bufs[key] = torch.empty((M, N), dtype=torch.float32, device=enc3.device)
-        out = bufs[key]
-        x2 = enc3.reshape(M, enc3.shape[-1])
-        if half:
-            torch.mm(x2, w["kv"][0].t(), out_dtype=torch.float32, out=out)
-        else:
-            prev = torch.backends.cuda.matmul.allow_tf32
-            torch.backends.cuda.matmul.allow_tf32 = True
-            try:
-                K = w["kv"][0].shape[1] // 3
-                torch.addmm(w["kv_bias"], x2[:, :K], w["kv"][0][:, :K].t(), out=out)
-                out.addmm_(x2[:, K:], w["kv"][0][:, K:].t())
-            finally:
-                torch.backends.cuda.matmul.allow_tf32 = prev
-        kv = out.view(enc3.shape[0], enc3.shape[1], n, 2, -1)
-        s = FP16_OUT_SCALE if half else 1.0
-        return [(kv[:, :, i, 0], kv[:, :, i, 1], s) for i in range(n)]
+        out = f.mm(enc3, kv, out=bufs[key]).view(enc3.shape[0], enc3.shape[1], n, 2, -1)
+        return [(out[:, :, i, 0], out[:, :, i, 1], f.scale) for i in range(n)]
 
-    USE_VIT_GRAPH = True
-
-    def _encode(self, imgs):
-        """(enc or None, per-block cross-attention (k, v) or [None]*n) for the current gemm_precision."""
-        mode = self.gemm_precision
-        if mode in self.SPLIT_MODES and imgs.is_cuda and not any(p.requires_grad for p in self.visual_encoder.parameters()):
-            with torch.no_grad():
-                if self.USE_VIT_GRAPH:
-                    kvs = self._encode_graphed(imgs, mode)
-                    if kvs is not None:
-                        return None, kvs
-                enc3, _ = self._vit3(imgs, mode=mode)
-                return None, self._cross_kv3(enc3, mode)
-        return self._vit(imgs), [None] * len(self.layer)
-
-    def _encode_graphed(self, imgs, mode):
-        """The encoder pass + the K/V GEMM replayed from a CUDA graph (one per image shape): ~330 launches whose host-side issue
-        otherwise leaves the GPU idle for ~3 ms per pass.  The graph's only output is the persistent K/V buffer of _cross_kv3.
-        Returns None when capture is impossible here."""
-        graphs = self.__dict__.setdefault("_vit_graphs", {})
-        self._weights3(mode)                       # (re)builds the splits when a weight changed ...
-        stamp = self.__dict__["_w3_cache"][mode]["stamp"]
-        key = (tuple(imgs.shape), str(imgs.device), mode)
-        ent = graphs.get(key)
-        if ent is not None and ent is not False and ent[2] != stamp:
-            ent = None                             # ... and a graph captured with the old splits is dropped
-        if ent is False:
-            return None
-        if ent is None:
-            static = imgs.clone()
+    def _graphed(self, key, what, inputs, run):
+        """run(*inputs) replayed from the CUDA graph kept under `key`, captured on first use after two warm-ups on a side stream
+        (autograd buffers, cuBLAS workspaces); `inputs` are copied into the graph's own copies of them.  -> run's result, which
+        the next replay overwrites, or None when capture failed (a warning, once per key; eager is always correct)."""
+        graphs = self._cache("graphs")
+        if key not in graphs:
+            static = [t.clone() for t in inputs]
             try:
                 cur = torch.cuda.current_stream()
                 side = torch.cuda.Stream()
                 side.wait_stream(cur)
                 with torch.cuda.stream(side):
                     for _ in range(2):
-                        self._cross_kv3(self._vit3(static, mode=mode)[0], mode)
+                        run(*static)
                 cur.wait_stream(side)
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g):
-                    kvs = self._cross_kv3(self._vit3(static, mode=mode)[0], mode)
-                ent = (g, static, stamp, kvs)
-            except Exception as e:  # noqa: BLE001 -- eager is always correct
+                    out = run(*static)
+                graphs[key] = (g, static, out)
+            except Exception as e:  # noqa: BLE001 -- a failed capture must not take the pass down
                 import warnings
-                warnings.warn("encoder CUDA graph capture failed (%s); running it eagerly" % str(e).splitlines()[0][:200])
+                warnings.warn("%s CUDA graph capture failed (%s); running it eagerly" % (what, str(e).partition("\n")[0][:200]))
                 torch.cuda.synchronize()
-                graphs[key] = False
-                return None
-            graphs[key] = ent
-        g, static, _, kvs = ent
-        static.copy_(imgs)
+                graphs[key] = None
+        if graphs[key] is None:
+            return None
+        g, static, out = graphs[key]
+        for s, t in zip(static, inputs):
+            s.copy_(t)
         g.replay()
-        return kvs
+        return out
+
+    USE_VIT_GRAPH = True
+
+    def _encode(self, imgs):
+        """(enc or None, per-block cross-attention (k, v, s) or [None]*n) for the current gemm_precision.  enc is None on the
+        split path: a split mode, CUDA input and frozen weights."""
+        mode = self.gemm_precision
+        if mode in self.SPLIT_MODES and imgs.is_cuda and self._refresh():
+            with torch.no_grad():
+                kvs = self._encode_graphed(imgs, mode) if self.USE_VIT_GRAPH else None
+                if kvs is None:
+                    kvs = self._cross_kv3(self._vit3(imgs, mode=mode)[0], mode)
+                return None, kvs
+        return self._vit(imgs), [None] * len(self.layer)
+
+    def _encode_graphed(self, imgs, mode):
+        """The encoder pass + the K/V GEMM replayed from a CUDA graph (one per image shape): ~330 launches whose host-side issue
+        otherwise leaves the GPU idle for ~3 ms per pass.  The graph's only output is the persistent K/V buffer of _cross_kv3.
+        Returns None when capture is impossible here."""
+        return self._graphed(("encoder", tuple(imgs.shape), str(imgs.device), mode), "encoder", (imgs,),
+                             lambda x: self._cross_kv3(self._vit3(x, mode=mode)[0], mode))
 
     def forward(self, visual_input, text_input=None, match_head="itm"):
         """ITM logits [B,2] (BITM:217-249, match_head='itm').  Also takes the LAVIS call form
@@ -561,28 +566,34 @@ class BlipITM(nn.Module):
         ids, att = self._tokenize(text_input, visual_input.device)
         enc, kvs = self._encode(visual_input)
         add_mask = ((1.0 - att.float()) * -10000.0)[:, None, None, :]
-        lin = self._text_linear()
+        lin = _plain_linear if enc is not None else self._linear3
         x = self._embed(ids)
         for lyr, kv in zip(self.layer, kvs):
             x = lyr.cross_and_ffn(lyr.self_attention(x, add_mask, lin), enc, kv, lin)
         return self.itm_head(x[:, 0])
 
-    def _text_pass(self, ids, add_mask, token_mask, enc, kvs, layer, head, cap):
+    def _text_pass(self, ids, add_mask, token_mask, enc, kvs, layer, head):
         """The text side of the trimmed GradCAM pass: BERT layers below `layer` without grad, the block's attention
         probabilities as the leaf, the loss differentiated w.r.t. them, the fused GradCAM kernel.  -> (cam [B,T-1,K-1], logits)."""
-        lin = self._text_linear()
-        with torch.no_grad():
-            x = self._embed(ids)
-            for lyr, kv in zip(self.layer[:layer], kvs):
-                x = lyr.cross_and_ffn(lyr.self_attention(x, add_mask, lin), enc, kv, lin)
-            x = self.layer[layer].self_attention(x, add_mask, lin)
-        with torch.enable_grad():
-            x = self.layer[layer].cross_and_ffn(x, enc, kvs[layer], lin)   # probs become a leaf inside (detach_probs)
-            for lyr, kv in zip(self.layer[layer + 1:], kvs[layer + 1:]):
-                x = lyr.cross_and_ffn(lyr.self_attention(x, add_mask, lin), enc, kv, lin)
-            out = self.itm_head(x[:, 0])
-            loss = out[:, 1].sum()
-            (dprobs,) = torch.autograd.grad(loss, cap.probs)
+        lin = _plain_linear if enc is not None else self._linear3
+        cap = GradcamCapture(head, token_mask)
+        xattn = self.layer[layer].crossattention.self
+        xattn.save_attention, xattn.capture, xattn.detach_probs = True, cap, True
+        try:
+            with torch.no_grad():
+                x = self._embed(ids)
+                for lyr, kv in zip(self.layer[:layer], kvs):
+                    x = lyr.cross_and_ffn(lyr.self_attention(x, add_mask, lin), enc, kv, lin)
+                x = self.layer[layer].self_attention(x, add_mask, lin)
+            with torch.enable_grad():
+                x = self.layer[layer].cross_and_ffn(x, enc, kvs[layer], lin)   # probs become a leaf inside (detach_probs)
+                for lyr, kv in zip(self.layer[layer + 1:], kvs[layer + 1:]):
+                    x = lyr.cross_and_ffn(lyr.self_attention(x, add_mask, lin), enc, kv, lin)
+                out = self.itm_head(x[:, 0])
+                loss = out[:, 1].sum()
+                (dprobs,) = torch.autograd.grad(loss, cap.probs)
+        finally:
+            xattn.save_attention, xattn.capture, xattn.detach_probs = False, None, False
         cap.dprobs = dprobs
         _, cam = ops.softmax_bwd_gradcam(cap.probs.detach(), dprobs.contiguous(), token_mask, head,
                                          1.0 / math.sqrt(64), need_dscores=False, need_gradcam=True)
@@ -594,57 +605,13 @@ class BlipITM(nn.Module):
     def _text_pass_graphed(self, ids, add_mask, token_mask, kvs, layer, head):
         """_text_pass replayed from a CUDA graph: the text side is ~700 launches of kernels that each run for microseconds
         (B*T = 875 rows at cfg1), so issued one by one it is bound by launch latency, not by the GPU.  One graph per
-        (shapes, block, head); inputs are copied into the graph's static buffers, the result is copied out.
+        (shapes, block, head); the K/V views of _cross_kv3's persistent buffer are read in place, the result is copied out.
         Returns None when capture is impossible here (the caller then runs the eager pass)."""
-        graphs = self.__dict__.setdefault("_text_graphs", {})
-        stamp = tuple(p._version for p in self.layer.parameters()) + tuple(p._version for p in self.itm_head.parameters())
-        if self.__dict__.get("_text_graph_stamp") != stamp:     # a graph holds the addresses of the weight splits it was captured with
-            graphs.clear()
-            self.__dict__["_text_graph_stamp"] = stamp
-        k0, v0, s0 = kvs[0]
-        key = (tuple(ids.shape), tuple(k0.shape), k0.data_ptr(), int(layer), int(head), float(s0), str(ids.device), token_mask.shape[1],
-               self.gemm_precision)
-        ent = graphs.get(key)
-        if ent is False:
-            return None
-        if ent is None:
-            st = {"ids": ids.clone(), "add_mask": add_mask.clone(), "token_mask": token_mask.clone()}
-            skvs = kvs                             # views of the persistent K/V buffer of _cross_kv3: fixed addresses
-            xattn = self.layer[layer].crossattention.self
-
-            def run():
-                cap = GradcamCapture(head, st["token_mask"])
-                xattn.save_attention, xattn.capture, xattn.detach_probs = True, cap, True
-                try:
-                    return self._text_pass(st["ids"], st["add_mask"], st["token_mask"], None, skvs, layer, head, cap)
-                finally:
-                    xattn.save_attention, xattn.capture, xattn.detach_probs = False, None, False
-
-            try:
-                cur = torch.cuda.current_stream()
-                side = torch.cuda.Stream()
-                side.wait_stream(cur)
-                with torch.cuda.stream(side):      # warm-up off the capture stream (autograd buffers, cuBLAS workspaces)
-                    for _ in range(2):
-                        run()
-                cur.wait_stream(side)
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g):
-                    st["cam"], st["out"] = run()
-                ent = (g, st)
-            except Exception as e:  # noqa: BLE001 -- a failed capture must not take the pass down; eager is always correct
-                import warnings
-                warnings.warn("text-pass CUDA graph capture failed (%s); running it eagerly" % str(e).splitlines()[0][:200])
-                torch.cuda.synchronize()
-                graphs[key] = False
-                return None
-            graphs[key] = ent
-        g, st = ent
-        st["ids"].copy_(ids)
-        st["add_mask"].copy_(add_mask)
-        st["token_mask"].copy_(token_mask)
-        g.replay()
-        return st["cam"].clone(), st["out"].clone()
+        k0, _, s0 = kvs[0]
+        key = ("text", tuple(ids.shape), tuple(k0.shape), k0.data_ptr(), int(layer), int(head), float(s0), str(ids.device),
+               token_mask.shape[1], self.gemm_precision)
+        res = self._graphed(key, "text-pass", (ids, add_mask, token_mask), lambda *st: self._text_pass(*st, None, kvs, layer, head))
+        return None if res is None else (res[0].clone(), res[1].clone())
 
     # ---- GradCAM of one (block, head) ----------------------------------------------------------------
     def gradcam(self, visual_input, text_input, tokenized_text, layer=7, head=9, full_backward=False):
@@ -656,12 +623,12 @@ class BlipITM(nn.Module):
         if token_mask.dtype != torch.int64:
             token_mask = token_mask.long()
         token_mask = token_mask.contiguous()
-        cap = GradcamCapture(head, token_mask)
-        xattn = self.layer[layer].crossattention.self
-        xattn.save_attention, xattn.capture, xattn.detach_probs = True, cap, not full_backward
         add_mask = ((1.0 - att.float()) * -10000.0)[:, None, None, :]
-        try:
-            if full_backward:
+        if full_backward:
+            cap = GradcamCapture(head, token_mask)
+            xattn = self.layer[layer].crossattention.self
+            xattn.save_attention, xattn.capture = True, cap
+            try:
                 with torch.enable_grad():
                     enc = self._vit(visual_input)
                     x = self._embed(ids)
@@ -671,15 +638,13 @@ class BlipITM(nn.Module):
                     loss = out[:, 1].sum()       # BITM:399
                     self.zero_grad()
                     loss.backward()              # BITM:404; FusedXattnSoftmax.backward fills cap.gradcam
-                cam = cap.gradcam
-            else:
-                with torch.no_grad():
-                    enc, kvs = self._encode(visual_input)
-                res = None
-                if self.USE_TEXT_GRAPH and enc is None and self._text_linear() is not _plain_linear:
-                    res = self._text_pass_graphed(ids, add_mask, token_mask, kvs, layer, head)
-                cam, out = res if res is not None else self._text_pass(ids, add_mask, token_mask, enc, kvs, layer, head, cap)
-        finally:
-            xattn.save_attention, xattn.capture, xattn.detach_probs = False, None, False
+            finally:
+                xattn.save_attention, xattn.capture = False, None
+            cam = cap.gradcam
+        else:
+            with torch.no_grad():
+                enc, kvs = self._encode(visual_input)
+            res = self._text_pass_graphed(ids, add_mask, token_mask, kvs, layer, head) if self.USE_TEXT_GRAPH and enc is None else None
+            cam, out = res if res is not None else self._text_pass(ids, add_mask, token_mask, enc, kvs, layer, head)
         P = self.patch_num
         return cam.view(B, T - 1, P, P), out.detach()

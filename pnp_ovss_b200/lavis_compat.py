@@ -116,8 +116,6 @@ def load_lavis_state_dict(model, state_dict):
             raise ValueError("%s: checkpoint shape %s, model shape %s" % (lk, tuple(t.shape), tuple(own[nk].shape)))
         new[nk] = t
     model.load_state_dict(new, strict=True)
-    for k in getattr(model, "_CACHES", ("_w3_cache",)):   # weight splits / captured graphs belong to the old weights
-        model.__dict__.pop(k, None)
     return ignored
 
 
