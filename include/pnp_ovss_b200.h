@@ -265,14 +265,17 @@ int pnp_layernorm_tf32_split3(const float *x, const float *residual, const float
  * [h * hi_scale | l | h] ([M,3K] halves).  Against a weight operand [W_h 2^b | W_h | W_l] with hi_scale * 2^b = 2^11, ONE fp16
  * tensor-core GEMM with fp32 accumulation yields 2^11 * (x W^T) at fp32-grade accuracy; the consumer takes the factor back
  * through in_scale / residual_scale (x is multiplied by in_scale before anything else; the residual by residual_scale).
- * *overflow_flag (device int, optional) is set to 1 when a value does not fit fp16 (|x| * hi_scale > 65504, inf or NaN):
- * the caller checks it once per run and falls back to the TF32 form.  K % 4 == 0; out3 8-byte aligned. */
+ * *overflow_flag (device int, optional) is set to 1, and never cleared, when a value does not fit fp16: when h * hi_scale,
+ * computed in fp16, is inf or NaN (so an x that rounds to fp16's largest value, 65504 / hi_scale, still fits; an inf or NaN x
+ * never does).  The caller checks it once per run and falls back to the TF32 form.  K % 4 == 0; out3 8-byte aligned. */
 int pnp_fp16_split3(const float *x, float in_scale, float hi_scale, uint16_t *out3, int *overflow_flag, long long M,
                     int K, pnp_stream_t stream);
 int pnp_gelu_fp16_split3(const float *x, float in_scale, const float *bias, float hi_scale, uint16_t *out3,
                          int *overflow_flag, long long M, int K, pnp_stream_t stream);
 /* ld_out3 = row stride of out3 in halves: 3K, or 3K + 8 to append the bias columns [bias_one, 1, 0 x 6] to every row -- against
- * the weight rows [b_h 2^11 / bias_one, b_l, 0 x 6] (b = b_h + b_l 2^-11) the GEMM then adds the layer's bias by itself. */
+ * the weight rows [b_h 2^11 / bias_one, b_l, 0 x 6] (b = b_h + b_l 2^-11) the GEMM then adds the layer's bias by itself.
+ * 3K + 8 needs K % 8 == 0 and a 16-byte aligned out3 (each row's bias columns are one 16-byte store).  Only out3 entries
+ * raise the overflow flag; out1 and x_out never do. */
 int pnp_layernorm_fp16_split3(const float *x, const float *residual, float residual_scale,
                               const float *residual_bias, float *x_out, const float *gamma, const float *beta,
                               float eps, float hi_scale, uint16_t *out3, int ld_out3, float bias_one, float *out1,

@@ -25,9 +25,11 @@
 namespace pnp {
 
 __device__ __forceinline__ float tf32_hi(float x) {
-    // round to nearest (ties away) at bit 13; non-finite inputs and overflow to inf keep x itself (lo = 0)
+    // round to nearest (ties away) at bit 13.  Where the carry would leave the finite range x is kept (lo = 0): from
+    // |x| = 0x1.ffep+127 (0x7F7FF000) up, +-inf, and NaN -- whose arithmetic form 0x7FFFFFFF would carry into the sign bit
+    // and round to -0
     float hi = __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xffffe000u);
-    return (fabsf(hi) <= 3.402823466e38f) ? hi : x;
+    return (fabsf(x) < 0x1.ffep+127f) ? hi : x;
 }
 
 // ---- operand writers.  kHalf == false: fp32 [hi | lo | hi] for the 3xTF32 GEMM; kHalf == true: fp16 [hi*2^a | lo*2^11 | hi]
@@ -164,16 +166,23 @@ __global__ void __launch_bounds__(256, kChunks <= 8 ? 3 : 1) layernorm_split3_ke
                 v[c] = make_float4(0.f, 0.f, 0.f, 0.f);
             }
         }
-        const float mean = warp_sum(sum) / (float)K;
-        float sq = 0.f;
+        // corrected two-pass moments: the second pass also sums the deviations from the fp32 mean m0; their mean r moves the
+        // mean to m0 + r and takes r^2 out of the variance.  On a (near-)constant row rstd is about rsqrt(eps), and it would
+        // otherwise multiply m0's rounding error into the output (3e-5 |gamma| for a row of 0.3 at K = 768, eps = 1e-6).
+        const float mean0 = warp_sum(sum) / (float)K;
+        float sq = 0.f, dev = 0.f;
 #pragma unroll
         for (int c = 0; c < kChunks; ++c) {
             if ((lane + 32 * c) * 4 < K) {
-                const float a = v[c].x - mean, b = v[c].y - mean, cc = v[c].z - mean, d = v[c].w - mean;
+                const float a = v[c].x - mean0, b = v[c].y - mean0, cc = v[c].z - mean0, d = v[c].w - mean0;
+                dev += (a + b) + (cc + d);
                 sq += (a * a + b * b) + (cc * cc + d * d);
             }
         }
-        const float rstd = rsqrtf(warp_sum(sq) / (float)K + eps);
+        dev = warp_sum(dev);
+        const float r = dev / (float)K;
+        const float mean = mean0 + r;
+        const float rstd = rsqrtf(fmaxf(warp_sum(sq) - dev * r, 0.f) / (float)K + eps);
 #pragma unroll
         for (int c = 0; c < kChunks; ++c) {
             const int k = (lane + 32 * c) * 4;
@@ -279,7 +288,9 @@ extern "C" int pnp_layernorm_fp16_split3(const float *x, const float *residual, 
                                          float *x_out, const float *gamma, const float *beta, float eps, float hi_scale,
                                          uint16_t *out3, int ld_out3, float bias_one, float *out1, int *overflow_flag, long long M,
                                          int K, pnp_stream_t stream) {
-    if (out3 && ld_out3 != 3 * K && (ld_out3 != 3 * K + 8 || !aligned16(out3))) return PNP_ERR_INVALID_ARGUMENT;
+    // the 8 bias columns of a row go out as one 16-byte store at half offset m (3K + 8) + 3K: 16-byte aligned for every m
+    // only when K % 8 == 0
+    if (out3 && ld_out3 != 3 * K && (ld_out3 != 3 * K + 8 || K % 8 || !aligned16(out3))) return PNP_ERR_INVALID_ARGUMENT;
     if (!x || !gamma || !beta || (!out3 && !out1) || M < 0 || K < 4 || K % 4 || K > 128 * 16 || !aligned16(x) ||
         (out3 && (reinterpret_cast<uintptr_t>(out3) & 7)) || (out1 && !aligned16(out1)) || !aligned16(gamma) || !aligned16(beta) ||
         (residual && !aligned16(residual)) || (residual_bias && (!residual || !aligned16(residual_bias))) ||

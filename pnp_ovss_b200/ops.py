@@ -466,6 +466,8 @@ def layernorm_fp16_split3(x, gamma, beta, eps, residual=None, residual_scale=1.0
             raise PnpError("residual_bias needs a residual and must be [K]")
     if not (split or plain):
         raise PnpError("nothing to compute")
+    if bias_one is not None and K % 8:
+        raise PnpError("bias columns need K %% 8 == 0, got K = %d" % K)
     ld3 = 3 * K + (8 if bias_one is not None else 0)
     out3 = torch.empty(x.shape[:-1] + (ld3,), dtype=torch.float16, device=x.device) if split else None
     out1 = torch.empty_like(x) if plain else None
