@@ -117,7 +117,12 @@ int pnp_threshold_upsample(const float *class_maps, float *out, void *workspace,
  * truncate=4, axis 0 then axis 1, float32 between passes) called per channel from DRV:1005-1011.
  * in, out [n_maps,H,W] (out may NOT alias in); minmax [n_maps,2] receives (min, max) of each blurred map
  * (NaN if the map holds a NaN).  normalize != 0 additionally rewrites out = (out-min)/(max-min) in place;
- * normalize == 0 leaves that to the consumer (pnp_crf_unary_from_maps folds it in). */
+ * normalize == 0 leaves that to the consumer (pnp_crf_unary_from_maps folds it in).
+ * Non-finite input reaches exactly the outputs it reaches in scipy: those within the radius lw = int(4 sigma + 0.5), the
+ * reflection included, are NaN where a NaN or both infinities are in reach and +-inf where one infinity is; a map that blurs
+ * to +inf everywhere reports (inf, inf).  Limit: lw <= 369 (pass V stages a column strip with its 2 lw halo rows in shared
+ * memory), i.e. a longer side of at most 1847 px at sigma = 0.05 max(H, W); a larger radius gets workspace_bytes 0 and
+ * PNP_ERR_INVALID_ARGUMENT, and nothing is written. */
 size_t pnp_gaussian_blur_workspace_bytes(int n_maps, int H, int W, double sigma);
 int pnp_gaussian_blur(const float *in, float *out, float *minmax, void *workspace, size_t workspace_bytes,
                       int n_maps, int H, int W, double sigma, int normalize, pnp_stream_t stream);
@@ -132,7 +137,9 @@ int pnp_gaussian_blur(const float *in, float *out, float *minmax, void *workspac
  * Upsample and blur are linear and separable, so a class channel is A_y m A_x^T with A = G_sigma U (H x P, W x P): no
  * full-resolution input or intermediate exists; Scale_0_1 is affine per channel and cancels in the min-max that follows
  * the blur, so `rescale` only enters the background test.  The background indicator is evaluated at full resolution with
- * the arithmetic of pnp_threshold_upsample and blurred tap by tap like pnp_gaussian_blur.  class_maps [B,C,P,P], P <= 32. */
+ * the arithmetic of pnp_threshold_upsample and blurred tap by tap like pnp_gaussian_blur, so with_background inherits that
+ * blur's limit (1847 px at sigma = 0.05 max(H, W)).  Without a background the fused kernels' own limits apply: lw <= 3007
+ * (about 15k px) and B, H <= 65535.  class_maps [B,C,P,P], P <= 32. */
 size_t pnp_lowrank_blur_workspace_bytes(int B, int C, int P, int H, int W, double sigma, int with_background);
 int pnp_lowrank_blur_unary(const float *class_maps, float *unary, int32_t *labels, float *maps_out, float *minmax_out,
                            void *workspace, size_t workspace_bytes, int B, int C, int P, int H, int W, float threshold,

@@ -217,6 +217,49 @@ __global__ void blur_prologue_kernel(float *__restrict__ weights, unsigned *__re
     }
 }
 
+// acc[r] += sum_j w[j] * v[(j + r) * kStride] over the taps = 2 lw + 1 taps, in chunks of 8 taps (one FMA order for every
+// pass and variant).  taps is odd, so the last chunk is partial: its padding taps (weight 0) are skipped rather than
+// multiplied, because the staged values they would meet are live data past the tap window, and 0 * NaN or 0 * inf would put
+// a NaN up to 7 px beyond the footprint of a non-finite input.  For finite data the result is the same bit for bit.
+// kWindowTail: the last chunk loads its sliding window once and predicates the FMAs (the loads of a full chunk; pass V), else
+// it runs tap by tap (16 loads a tap, but fewer live registers: the paired pass-H kernel, capped at 40, spills the window).
+// Measured on a B200 (profiles/time_blur_passes.py, DESIGN.md section 5), tap by tap is also the faster tail for both pass-H
+// kernels.
+template <int R, int kStride, bool kWindowTail>
+__device__ __forceinline__ void blur_taps(float (&acc)[R], const float *__restrict__ v, const float *__restrict__ w, int taps) {
+    int jc = 0;
+    for (; jc + 8 <= taps; jc += 8) {
+        float vv[R + 7], ww[8];
+#pragma unroll
+        for (int i = 0; i < R + 7; ++i) vv[i] = v[(jc + i) * kStride];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) ww[i] = w[jc + i];
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+#pragma unroll
+            for (int r = 0; r < R; ++r) acc[r] = fmaf(ww[i], vv[i + r], acc[r]);
+    }
+    if (kWindowTail) {   // the last 1..7 taps
+        const int rem = taps - jc;
+        float vv[R + 6], ww[7];
+#pragma unroll
+        for (int i = 0; i < R + 6; ++i) vv[i] = v[(jc + i) * kStride];
+#pragma unroll
+        for (int i = 0; i < 7; ++i) ww[i] = w[jc + i];
+#pragma unroll
+        for (int i = 0; i < 7; ++i)
+            if (i < rem)
+#pragma unroll
+                for (int r = 0; r < R; ++r) acc[r] = fmaf(ww[i], vv[i + r], acc[r]);
+        return;
+    }
+    for (; jc < taps; ++jc) {   // the last 1..7 taps, one at a time
+        const float wj = w[jc];
+#pragma unroll
+        for (int r = 0; r < R; ++r) acc[r] = fmaf(wj, v[(jc + r) * kStride], acc[r]);
+    }
+}
+
 constexpr int kVCols = 64;   // columns per CTA in pass V
 constexpr int kVRows = 16;   // output rows per thread per sweep
 constexpr int kVGroups = 8;  // row groups per CTA (kVCols * kVGroups = 512 threads)
@@ -250,17 +293,7 @@ __global__ void __launch_bounds__(kVCols *kVGroups) blur_vertical_kernel(const f
         float acc[kVRows];
 #pragma unroll
         for (int r = 0; r < kVRows; ++r) acc[r] = 0.f;
-        for (int jc = 0; jc < 2 * lw + 1; jc += 8) {
-            float vv[kVRows + 7], ww[8];
-#pragma unroll
-            for (int i = 0; i < kVRows + 7; ++i) vv[i] = s_in[(yl + jc + i) * kVCols + cx];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) ww[i] = s_w[jc + i];
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-#pragma unroll
-                for (int r = 0; r < kVRows; ++r) acc[r] = fmaf(ww[i], vv[i + r], acc[r]);
-        }
+        blur_taps<kVRows, kVCols, true>(acc, s_in + yl * kVCols + cx, s_w, 2 * lw + 1);
         if (gx < W) {
 #pragma unroll
             for (int r = 0; r < kVRows; ++r)
@@ -339,17 +372,7 @@ __global__ void __launch_bounds__(kTCols *kTGroups) blur_vertical_tma_kernel(con
         float acc[kVRows];
 #pragma unroll
         for (int r = 0; r < kVRows; ++r) acc[r] = 0.f;
-        for (int jc = 0; jc < 2 * lw + 1; jc += 8) {
-            float vv[kVRows + 7], ww[8];
-#pragma unroll
-            for (int i = 0; i < kVRows + 7; ++i) vv[i] = s_in[(yl + jc + i) * kTCols + cx];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) ww[i] = s_w[jc + i];
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-#pragma unroll
-                for (int r = 0; r < kVRows; ++r) acc[r] = fmaf(ww[i], vv[i + r], acc[r]);
-        }
+        blur_taps<kVRows, kTCols, true>(acc, s_in + yl * kTCols + cx, s_w, 2 * lw + 1);
         if (gx < W) {
 #pragma unroll
             for (int r = 0; r < kVRows; ++r)
@@ -395,25 +418,14 @@ __global__ void __launch_bounds__(kHRows *kMaxWarps, kMinCtas) blur_horizontal_k
     const int lane = threadIdx.x & 31, grp = threadIdx.x >> 5;
     const int gy = y_base + lane;
     float mn = INFINITY, mx = -INFINITY;
-    bool has_nan = false;
+    bool has_nan = false, seen = false;   // seen: this thread wrote a pixel (mn == inf also means a map of +inf)
     for (int sweep = 0; sweep < cols_here; sweep += n_groups * kHCols) {
         const int xl = sweep + grp * kHCols;
         if (xl < cols_here) {
             float acc[kHCols];
 #pragma unroll
             for (int r = 0; r < kHCols; ++r) acc[r] = 0.f;
-            const float *row = s_in + lane * pitch + xl;
-            for (int jc = 0; jc < 2 * lw + 1; jc += 8) {
-                float vv[kHCols + 7], ww[8];
-#pragma unroll
-                for (int i = 0; i < kHCols + 7; ++i) vv[i] = row[jc + i];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) ww[i] = s_w[jc + i];
-#pragma unroll
-                for (int i = 0; i < 8; ++i)
-#pragma unroll
-                    for (int r = 0; r < kHCols; ++r) acc[r] = fmaf(ww[i], vv[i + r], acc[r]);
-            }
+            blur_taps<kHCols, 1, false>(acc, s_in + lane * pitch + xl, s_w, 2 * lw + 1);
 #pragma unroll
             for (int r = 0; r < kHCols; ++r) s_out[lane * kOutPitch + grp * kHCols + r] = acc[r];
         }
@@ -425,6 +437,7 @@ __global__ void __launch_bounds__(kHRows *kMaxWarps, kMinCtas) blur_horizontal_k
             if (y_base + r < H) {
                 float v = s_out[r * kOutPitch + c];
                 dst[(long long)(y_base + r) * W + x_base + sweep + c] = v;
+                seen = true;
                 has_nan = has_nan || (v != v);
                 mn = fminf(mn, v);
                 mx = fmaxf(mx, v);
@@ -434,7 +447,7 @@ __global__ void __launch_bounds__(kHRows *kMaxWarps, kMinCtas) blur_horizontal_k
     }
     (void)gy;
     unsigned kmin = has_nan ? 0u : f2key(mn), kmax = has_nan ? 0xffffffffu : f2key(mx);
-    if (mn == INFINITY && !has_nan) { kmin = 0xffffffffu; kmax = 0u; }  // thread saw no pixel
+    if (!seen) { kmin = 0xffffffffu; kmax = 0u; }
     for (int o = 16; o > 0; o >>= 1) {
         kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, o));
         kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, o));
@@ -857,15 +870,21 @@ extern "C" int pnp_gaussian_blur(const float *in, float *out, float *minmax, voi
 // ------------------------------------------------------------------------------------------------ fused low-rank entry point
 namespace {
 struct LowrankPlan {
-    BlurPlan blur;   // direct blur of the B background maps
-    int PPAD, rows_chunk, threads_a, tile_pix;
+    BlurPlan blur;   // direct blur of the B background maps (planned only with_background)
+    int lw, PPAD, rows_chunk, threads_a, tile_pix;
     size_t smem_a, smem_b;
     size_t off_masked, off_params, off_ay, off_axt, off_T, off_norm, off_bg, off_bgblur, off_bgmm, off_blur_ws, total;
 };
 
 bool make_lowrank_plan(int B, int C, int P, int H, int W, double sigma, int with_background, LowrankPlan &p) {
-    if (B < 0 || C < 1 || P < 1 || P > kLrMaxP || H < 1 || W < 1) return false;
-    if (!make_blur_plan(with_background ? B : 0, H, W, sigma, p.blur)) return false;
+    if (B < 0 || C < 1 || P < 1 || P > kLrMaxP || H < 1 || W < 1 || !(sigma > 0.0)) return false;
+    // only the background maps take the direct blur: without them its size limits do not apply
+    p.blur = BlurPlan{};
+    if (with_background && !make_blur_plan(B, H, W, sigma, p.blur)) return false;
+    // lowrank_operator_kernel keeps the 2 lw + 1 float64 weights in dynamic shared memory, next to its 1 KB s_part, within the
+    // 48 KB a CTA gets without opting in: lw <= 3007
+    if (!(4.0 * sigma + 0.5 < (48 * 1024 - 128 * sizeof(double)) / (2 * sizeof(double)))) return false;
+    p.lw = blur_radius(sigma);
     p.PPAD = P <= 24 ? 24 : (P <= 28 ? 28 : 32);
     p.rows_chunk = std::min(H, 512);   // <= 64 KB of T per chunk
     {   // pass A: one thread per column, as few sweeps over x as possible
@@ -947,8 +966,8 @@ extern "C" int pnp_lowrank_blur_unary_padded(const float *class_maps, const int3
     // reference's rescale silently does not happen (DRV:1079-1080), as in pnp_threshold_upsample
     const int bg_rescale = (rescale && with_background && (n_classes || C > 1)) ? 1 : 0;   // per image in the kernels when n_classes is given
     char *bws = ws + p.off_blur_ws;
-    lowrank_operator_kernel<<<ceil_div(H + W, 128), 128, (2 * p.blur.lw + 1) * sizeof(double), st>>>(
-        reinterpret_cast<float *>(ws + p.off_ay), reinterpret_cast<float *>(ws + p.off_axt), H, W, P, p.PPAD, p.blur.lw, sigma);
+    lowrank_operator_kernel<<<ceil_div(H + W, 128), 128, (2 * p.lw + 1) * sizeof(double), st>>>(
+        reinterpret_cast<float *>(ws + p.off_ay), reinterpret_cast<float *>(ws + p.off_axt), H, W, P, p.PPAD, p.lw, sigma);
     PNP_LAUNCH(kThresholdPrep, st, threshold_prep_kernel<<<dim3(C, B), 256, 0, st>>>(class_maps, masked, params, C, P, H, W, threshold, bg_rescale, n_classes));
     int rc = launch_status();
     if (rc != PNP_OK) return rc;
