@@ -184,10 +184,15 @@ typedef struct pnp_lattice {
     int32_t *counters; /* [8] device: 0 = M, 1 = key-range overflow flag, 2 = longest row */
 } pnp_lattice;
 
-/* Bytes of persistent storage a lattice needs, and of scratch needed while building it. */
+/* Bytes of persistent storage a lattice needs, and of scratch needed while building it; 0 for a refused shape.
+ * A shape is refused unless d is 2 or 5, n_images*n_pixels*(d+1) < 0x7f000000, and n_images*capacity <= INT32_MAX, where
+ * capacity, the hash-table slots of one image, is 2*n_pixels*(d+1) rounded up to a power of two (at least 1024): the build
+ * indexes the slots of all images with one int32.  So at d = 5 a batch holds at most 511 images of 512x512 or 1023 of
+ * 336x336, and at d = 2 at most 1023 of 512x512. */
 size_t pnp_lattice_storage_bytes(int d, int n_images, int n_pixels);
 size_t pnp_lattice_build_workspace_bytes(int d, int n_images, int n_pixels);
-/* Carve `storage` (device, >= pnp_lattice_storage_bytes, 256-byte aligned) into the arrays of *lat (host). */
+/* Carve `storage` (device, >= pnp_lattice_storage_bytes, 256-byte aligned) into the arrays of *lat (host).
+ * PNP_ERR_INVALID_ARGUMENT for a refused shape (above); it touches no device memory. */
 int pnp_lattice_init(pnp_lattice *lat, void *storage, size_t storage_bytes, int d, int n_images, int n_pixels,
                      int shared);
 /* Enqueue the whole build: embed pixels (elevate, round, rank, barycentric), hash-insert the d+1 simplex

@@ -505,9 +505,9 @@ __global__ void __launch_bounds__(256) csr_norm_fill_kernel(const int32_t *__res
 }
 
 // ------------------------------------------------------------------------------------------ host side
-static inline unsigned table_capacity(int d, int n_pixels) {
+static inline unsigned long long table_capacity(int d, int n_pixels) {
     unsigned long long need = 2ull * (unsigned long long)n_pixels * (d + 1);
-    unsigned cap = 1024;
+    unsigned long long cap = 1024;
     while (cap < need) cap <<= 1;
     return cap;
 }
@@ -542,8 +542,16 @@ static BuildLayout build_layout(int d, int n_images, int n_pixels) {
 
 using namespace pnp;
 
+// The build addresses the hash tables of all images as one int32 slot index (img * capacity + h in lattice_embed_kernel and
+// lattice_neighbors_kernel), and numbers entries with int32 ids below the 0x7f7f7f7f fill of `first`.
+static bool lattice_shape_ok(int d, int n_images, int n_pixels) {
+    if ((d != 2 && d != 5) || n_images < 1 || n_pixels < 1) return false;
+    if ((size_t)n_images * n_pixels * (d + 1) >= 0x7f000000ull) return false;
+    return (unsigned long long)n_images * table_capacity(d, n_pixels) <= 0x7fffffffull;
+}
+
 extern "C" size_t pnp_lattice_storage_bytes(int d, int n_images, int n_pixels) {
-    if ((d != 2 && d != 5) || n_images < 1 || n_pixels < 1) return 0;
+    if (!lattice_shape_ok(d, n_images, n_pixels)) return 0;
     const size_t n_entries = (size_t)n_images * n_pixels * (d + 1);
     size_t o = 0;
     o += align_up(n_entries * 4, 256);                        // offset
@@ -559,17 +567,16 @@ extern "C" size_t pnp_lattice_storage_bytes(int d, int n_images, int n_pixels) {
 }
 
 extern "C" size_t pnp_lattice_build_workspace_bytes(int d, int n_images, int n_pixels) {
-    if ((d != 2 && d != 5) || n_images < 1 || n_pixels < 1) return 0;
+    if (!lattice_shape_ok(d, n_images, n_pixels)) return 0;
     return build_layout(d, n_images, n_pixels).total;
 }
 
 extern "C" int pnp_lattice_init(pnp_lattice *lat, void *storage, size_t storage_bytes, int d, int n_images, int n_pixels,
                                 int shared) {
-    if (!lat || !storage || (d != 2 && d != 5) || n_images < 1 || n_pixels < 1) return PNP_ERR_INVALID_ARGUMENT;
+    if (!lat || !storage || !lattice_shape_ok(d, n_images, n_pixels)) return PNP_ERR_INVALID_ARGUMENT;
     if (shared && n_images != 1) return PNP_ERR_INVALID_ARGUMENT;
     if ((reinterpret_cast<uintptr_t>(storage) & 255) != 0) return PNP_ERR_INVALID_ARGUMENT;
     const size_t n_entries = (size_t)n_images * n_pixels * (d + 1);
-    if (n_entries >= 0x7f000000ull) return PNP_ERR_INVALID_ARGUMENT;  // entry ids are int32 and < the 0x7f7f7f7f fill of `first`
     if (storage_bytes < pnp_lattice_storage_bytes(d, n_images, n_pixels)) return PNP_ERR_WORKSPACE;
     char *p = reinterpret_cast<char *>(storage);
     auto take = [&](size_t bytes) { char *r = p; p += align_up(bytes, 256); return r; };
@@ -600,7 +607,7 @@ static int build_impl(pnp_lattice *lat, const uint8_t *rgb, int H, int W, float 
     const long long n_lp = (long long)lat->n_images * N;
     const long long n_entries = n_lp * (D + 1);
     const BuildLayout L = build_layout(D, lat->n_images, N);
-    const unsigned cap = table_capacity(D, N);
+    const unsigned cap = (unsigned)table_capacity(D, N);  // n_images * cap <= INT32_MAX (lattice_shape_ok)
     const size_t slots = (size_t)lat->n_images * cap;
     auto *table = reinterpret_cast<unsigned long long *>(ws + L.off_table);
     auto *first = reinterpret_cast<int32_t *>(ws + L.off_first);
@@ -675,7 +682,9 @@ extern "C" int pnp_lattice_build(pnp_lattice *lat, const uint8_t *rgb, int H, in
     if (!(sx > 0.f) || !(sy > 0.f)) return PNP_ERR_INVALID_ARGUMENT;
     if ((lat->d == 5) != (rgb != nullptr)) return PNP_ERR_INVALID_ARGUMENT;
     if (lat->d == 5 && (!(sr > 0.f) || !(sg > 0.f) || !(sb > 0.f))) return PNP_ERR_INVALID_ARGUMENT;
-    if (workspace_bytes < pnp_lattice_build_workspace_bytes(lat->d, lat->n_images, lat->n_pixels)) return PNP_ERR_WORKSPACE;
+    const size_t need = pnp_lattice_build_workspace_bytes(lat->d, lat->n_images, lat->n_pixels);
+    if (need == 0) return PNP_ERR_INVALID_ARGUMENT;
+    if (workspace_bytes < need) return PNP_ERR_WORKSPACE;
     if ((reinterpret_cast<uintptr_t>(workspace) & 255) != 0) return PNP_ERR_INVALID_ARGUMENT;
     char *ws = reinterpret_cast<char *>(workspace);
     lat->width = W;

@@ -233,7 +233,7 @@ class LatticeHandle:
         return self.storage[off:off + count * itemsize].view(dtype)
 
     def arrays(self):
-        """Device views (for tests): offset [n_lp,d+1], bary, nbr [d+1,M,2], norm [n_lp], row_ptr, csr_pix, csr_w."""
+        """Device views (for tests): offset [n_lp,d+1], bary, nbr [d+1,M,2], norm [n_lp], row_ptr, csr_pix, csr_w, csr_norm."""
         s = self.struct
         n_lp = s.n_images * s.n_pixels
         D1 = s.d + 1
@@ -246,6 +246,7 @@ class LatticeHandle:
             "row_ptr": self._view("row_ptr", s.n_vertices + 1, torch.int32),
             "csr_pix": self._view("csr_pix", ne, torch.int32),
             "csr_w": self._view("csr_w", ne, torch.float32),
+            "csr_norm": self._view("csr_norm", ne, torch.float32),
         }
 
 
