@@ -252,6 +252,16 @@ int pnp_confusion_accumulate(const int32_t *labels, const float *gt, const int32
                              float *pred_out, int64_t *hist, int32_t *bad_count, int B, int N, int n_class,
                              pnp_stream_t stream);
 
+/* The same relabel without ground truth, for images that have none (the in-the-wild output):
+ *   ids_out[b,n]  = lut[b, labels[b,n]]
+ *   conf_out[b,n] = Q[b,n, labels[b,n]]  (the CRF marginal of the chosen label; Q [B,N,Cp] pixel-major as pnp_crf_inference
+ *                                         writes it)
+ * labels int32 [B,N]; lut int32 [B,lut_stride]; ids_out int32 [B,N].  Q and conf_out are optional, both NULL or both non-NULL,
+ * and then Cp >= lut_stride.  A label outside [0, lut_stride) writes -1 to ids_out (and to conf_out) and reads nothing.
+ * The in-situ profiler times it with the relabel stage it replaces, kernel class 16 (confusion). */
+int pnp_label_map(const int32_t *labels, const int32_t *lut, int lut_stride, const float *Q, int Cp, int32_t *ids_out,
+                  float *conf_out, int B, int N, pnp_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * (f)1 model pass (SURVEY 8f.1; BITM:386-404 drives VIT:93-119 / MED:201-228): operand preparation for
  *      fp32-grade GEMMs on the TF32 tensor cores.  The dense contractions themselves stay torch's (cuBLAS);

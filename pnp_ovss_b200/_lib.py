@@ -80,6 +80,7 @@ SIGNATURES = {
     "pnp_argmax_channels": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "pnp_confusion_accumulate": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                          c_int, c_void_p]),
+    "pnp_label_map": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p]),
 }
 
 _lib = None

@@ -137,6 +137,53 @@ __global__ void __launch_bounds__(512) confusion_kernel(const int32_t *__restric
     }
 }
 
+// ------------------------------------------------------------------ label map + confidence (no ground truth)
+// ids[p] = lut[b, labels[p]], conf[p] = Q[p, labels[p]] (Q pixel-major [B,N,Cp]); a label outside [0, lut_stride) gives -1 in
+// both.  kVec: N % 4 == 0 and 16-byte aligned labels / ids / conf -> four consecutive pixels of one image per thread, one
+// 128-bit streaming load of labels and one 128-bit store per output.  The lut and Q reads are gathers (one word per pixel).
+// Timed by the in-situ profiler as the relabel stage it stands in for (kConfusion).
+__device__ __forceinline__ void label_one(int lab, long long b, long long pix, const int32_t *__restrict__ lut, int lut_stride,
+                                          const float *__restrict__ Q, int Cp, int &id, float &conf) {
+    id = -1;
+    conf = -1.f;
+    if (lab >= 0 && lab < lut_stride) {
+        id = __ldg(lut + b * lut_stride + lab);
+        if (Q) conf = __ldg(Q + pix * Cp + lab);
+    }
+}
+
+template <bool kVec>
+__global__ void __launch_bounds__(256) label_map_kernel(const int32_t *__restrict__ labels, const int32_t *__restrict__ lut,
+                                                        int lut_stride, const float *__restrict__ Q, int Cp,
+                                                        int32_t *__restrict__ ids_out, float *__restrict__ conf_out, int N,
+                                                        long long total) {
+    constexpr int V = kVec ? 4 : 1;
+    const long long items = total / V;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < items; i += (long long)gridDim.x * blockDim.x) {
+        const long long p0 = i * V;
+        const long long b = p0 / N;   // N % V == 0: the V pixels of an item belong to one image
+        int lab[V], id[V];
+        float conf[V];
+        if (kVec) {   // int32 moved through the f32 streaming load / store: bit patterns pass unchanged
+            const float4 l4 = ldg_stream4(reinterpret_cast<const float *>(labels) + p0);
+            lab[0] = __float_as_int(l4.x); lab[V > 1 ? 1 : 0] = __float_as_int(l4.y);
+            lab[V > 2 ? 2 : 0] = __float_as_int(l4.z); lab[V > 3 ? 3 : 0] = __float_as_int(l4.w);
+        } else {
+            lab[0] = __ldg(labels + p0);
+        }
+#pragma unroll
+        for (int v = 0; v < V; ++v) label_one(lab[v], b, p0 + v, lut, lut_stride, Q, Cp, id[v], conf[v]);
+        if (kVec) {
+            stg_stream4(reinterpret_cast<float *>(ids_out) + p0, make_float4(__int_as_float(id[0]), __int_as_float(id[V > 1 ? 1 : 0]),
+                                                                              __int_as_float(id[V > 2 ? 2 : 0]), __int_as_float(id[V > 3 ? 3 : 0])));
+            if (conf_out) stg_stream4(conf_out + p0, make_float4(conf[0], conf[V > 1 ? 1 : 0], conf[V > 2 ? 2 : 0], conf[V > 3 ? 3 : 0]));
+        } else {
+            ids_out[p0] = id[0];
+            if (conf_out) conf_out[p0] = conf[0];
+        }
+    }
+}
+
 }  // namespace pnp
 
 using namespace pnp;
@@ -188,5 +235,24 @@ extern "C" int pnp_confusion_accumulate(const int32_t *labels, const float *gt, 
         else
             PNP_LAUNCH(kConfusion, st, (confusion_kernel<false, false><<<grid, 512, 0, st>>>(labels, gt, lut, lut_stride, pred_out, h, bad_count, N, total, n_class)));
     }
+    return launch_status();
+}
+
+extern "C" int pnp_label_map(const int32_t *labels, const int32_t *lut, int lut_stride, const float *Q, int Cp, int32_t *ids_out,
+                             float *conf_out, int B, int N, pnp_stream_t stream) {
+    if (!labels || !lut || !ids_out || lut_stride < 1 || B < 0 || N < 1) return PNP_ERR_INVALID_ARGUMENT;
+    if ((Q == nullptr) != (conf_out == nullptr)) return PNP_ERR_INVALID_ARGUMENT;
+    if (Q && Cp < lut_stride) return PNP_ERR_INVALID_ARGUMENT;   // every label the lut accepts must be a channel of Q
+    if (B == 0) return PNP_OK;
+    cudaStream_t st = as_stream(stream);
+    auto aligned = [](const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+    const bool vec = (N % 4 == 0) && aligned(labels) && aligned(ids_out) && (!conf_out || aligned(conf_out));
+    const long long total = (long long)B * N;
+    const long long items = vec ? total / 4 : total;
+    const int grid = (int)std::max<long long>(1, std::min<long long>((long long)kNumSMs * 16, (items + 255) / 256));
+    if (vec)
+        PNP_LAUNCH(kConfusion, st, (label_map_kernel<true><<<grid, 256, 0, st>>>(labels, lut, lut_stride, Q, Cp, ids_out, conf_out, N, total)));
+    else
+        PNP_LAUNCH(kConfusion, st, (label_map_kernel<false><<<grid, 256, 0, st>>>(labels, lut, lut_stride, Q, Cp, ids_out, conf_out, N, total)));
     return launch_status();
 }

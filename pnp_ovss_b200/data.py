@@ -89,12 +89,13 @@ def image_path(args, img_id):
 
 def load_model_image(path, img_size):
     """DS:430-443: (model input float32 [3,S,S], norm_img float32 [S,S,3] in 0..1, original (width, height)).
+    `path` is an image file, or an RGB image already decoded into a uint8 [H,W,3] array.
 
     The model input is the image resized to SxS with PIL's bicubic filter, scaled to 0..1 and normalised with the CLIP
     statistics (torchvision Resize(BICUBIC) -> ToTensor -> Normalize on a PIL image is exactly that); norm_img is the
     default-filter resize the reference keeps for its visualisations and the DropOut bookkeeping."""
     from PIL import Image
-    img0 = Image.open(path).convert("RGB")
+    img0 = Image.fromarray(path, "RGB") if isinstance(path, np.ndarray) else Image.open(path).convert("RGB")
     S = int(img_size)
     norm_img = np.float32(img0.resize((S, S))) / 255
     x = np.array(img0.resize((S, S), Image.BICUBIC), dtype=np.uint8)

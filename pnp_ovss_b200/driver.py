@@ -18,8 +18,18 @@ With the real inputs on disk the same driver runs them (`main_real`):
     python -m pnp_ovss_b200.driver --real_data --home_dir /data --data_type voc --bert_vocab vocab.txt \\
         --checkpoint model_large_retrieval_flickr.pth --img_size 336 --batch_size 35 --max_att_block_num 8 ...
 reads {home_dir}/VOCdevkit/VOC2012/{val.txt,JPEGImages,SegmentationClass} and {home_dir}/GPT4o_classification/*.json in the
-reference's layouts (pnp_ovss_b200/data.py, reference_api.save_img_union_attention)."""
+reference's layouts (pnp_ovss_b200/data.py, reference_api.save_img_union_attention).
+
+`--in_the_wild` segments your own images with class names you choose, without ground truth (segment.segment_images):
+    python -m pnp_ovss_b200.driver --in_the_wild --image_dir photos/ --classes "cat,dog,grass" --save_path out/ \
+        --img_size 336 --batch_size 35 --max_att_block_num 8 --prune_att_head 9 --drop_iter 4 --threshold 0.15 \
+        --postprocess blur+crf [--bert_vocab vocab.txt --checkpoint model_large_retrieval_flickr.pth]
+(`--class_file map.json` instead of --classes: a JSON object {image stem: [class names] or "a,b,c"}).  It writes
+out/in_the_wild/<stem>.png (a palette PNG: 0 = background, i = the i-th class of the image), <stem>_conf.npy (float32, the CRF
+marginal of each chosen label; modes with a CRF only) and classes.json ({stem: class list}).  Ranks take contiguous shards of
+the images in name order and write their own files.  An image the blur cannot take is refused with the reason and skipped."""
 import argparse
+import json
 import os
 import time
 
@@ -83,6 +93,10 @@ def get_args_parser():
                              "activations leave fp16's range is repeated in 3xtf32.")
     parser.add_argument("--synthetic_gt_size", default=0, type=int,
                         help="side of the ground-truth / guide images (0 = img_size); the maps are upsampled to it (DRV:435-437)")
+    parser.add_argument("--image_dir", default=None, type=str, help="--in_the_wild: the folder of images to segment")
+    parser.add_argument("--classes", default=None, type=str, help="--in_the_wild: comma-separated class names for every image")
+    parser.add_argument("--class_file", default=None, type=str,
+                        help="--in_the_wild: JSON object {image stem: [class names] or 'a,b,c'} (instead of --classes)")
     return parser
 
 
@@ -192,8 +206,142 @@ def main_real(rank, world_size, args, model=None):
     return result
 
 
+IMAGE_SUFFIXES = (".jpg", ".jpeg", ".png", ".bmp", ".tif", ".tiff", ".webp")
+
+
+def wild_images(image_dir):
+    """{stem: path} of the image files directly under image_dir.  Two files with one stem are refused: their outputs would
+    share a name."""
+    paths = {}
+    for name in sorted(os.listdir(image_dir)):
+        stem, ext = os.path.splitext(name)
+        if ext.lower() in IMAGE_SUFFIXES and os.path.isfile(os.path.join(image_dir, name)):
+            if stem in paths:
+                raise SystemExit("--image_dir holds two images with the stem %r (%s, %s)" % (stem, os.path.basename(paths[stem]), name))
+            paths[stem] = os.path.join(image_dir, name)
+    if not paths:
+        raise SystemExit("no image (%s) in --image_dir %s" % (", ".join(IMAGE_SUFFIXES), image_dir))
+    return paths
+
+
+def parse_class_names(text):
+    """'cat, dog,grass' -> ['cat', 'dog', 'grass']."""
+    return [c.strip() for c in text.split(",") if c.strip()]
+
+
+def wild_class_lists(args, stems):
+    """{stem: class names} from --classes (one list for every image) or --class_file; at least 1 and at most 255 classes per
+    image (the label PNG is 8-bit with 0 for the background)."""
+    if bool(args.classes) == bool(args.class_file):
+        raise SystemExit("--in_the_wild needs exactly one of --classes and --class_file")
+    if args.classes:
+        names = parse_class_names(args.classes)
+        out = {s: list(names) for s in stems}
+    else:
+        with open(args.class_file, "r") as f:
+            table = json.load(f)
+        if not isinstance(table, dict):
+            raise SystemExit("--class_file must hold a JSON object {image stem: [class names] or 'a,b,c'}")
+        missing = [s for s in stems if s not in table]
+        if missing:
+            raise SystemExit("--class_file has no classes for %s" % ", ".join(missing))
+        out = {s: parse_class_names(table[s]) if isinstance(table[s], str) else [str(c).strip() for c in table[s] if str(c).strip()]
+               for s in stems}
+    for s, names in out.items():
+        if not 1 <= len(names) <= 255:
+            raise SystemExit("image %s: %d classes (1 to 255 fit the 8-bit label map)" % (s, len(names)))
+    return out
+
+
+def wild_outputs(save_path, stem):
+    """(label PNG, confidence .npy) that --in_the_wild writes for one image."""
+    d = os.path.join(save_path, "in_the_wild")
+    return os.path.join(d, stem + ".png"), os.path.join(d, stem + "_conf.npy")
+
+
+def label_palette():
+    """The PASCAL VOC colour map (index 0 black): 768 palette bytes."""
+    pal = []
+    for i in range(256):
+        r = g = b = 0
+        c = i
+        for j in range(8):
+            r |= (c & 1) << (7 - j)
+            g |= ((c >> 1) & 1) << (7 - j)
+            b |= ((c >> 2) & 1) << (7 - j)
+            c >>= 3
+        pal += [r, g, b]
+    return pal
+
+
+def write_label_png(path, ids):
+    from PIL import Image
+    im = Image.fromarray(np.ascontiguousarray(ids, dtype=np.uint8))
+    im.putpalette(label_palette())
+    im.save(path)
+
+
+def main_in_the_wild(rank, world_size, args, model=None):
+    """--in_the_wild: segment_images over this rank's shard of --image_dir, files written per image (no collective).  A 3xFP16
+    run whose activations left fp16's range is repeated in 3xTF32 and overwrites its files.  Returns the stems this rank wrote."""
+    from .blip_itm import BlipITM
+    from .segment import image_size, segment_images, size_refusal
+    if args.image_dir is None or args.threshold is None or args.prune_att_head is None:
+        raise SystemExit("--in_the_wild needs --image_dir, --threshold and --prune_att_head")
+    data_type = args.data_type or "voc"
+    paths = wild_images(args.image_dir)
+    classes = wild_class_lists(args, list(paths))
+    stems = []
+    for s in paths:
+        why = size_refusal(*image_size(paths[s]), len(classes[s]), args.postprocess, data_type)
+        if why:
+            if rank == 0:
+                print("refused %s: %s" % (paths[s], why))
+        else:
+            stems.append(s)
+    torch.cuda.set_device(rank)
+    dev = torch.device("cuda", rank)
+    if model is None:
+        tok = data.init_tokenizer(args.bert_vocab) if args.bert_vocab else synthetic.SyntheticWordPieceTokenizer()
+        torch.manual_seed(4321)
+        model = BlipITM(img_size=int(args.img_size), tokenizer=tok).eval()
+        if args.checkpoint:
+            model.load_lavis_checkpoint(args.checkpoint)
+        model = model.to(dev).requires_grad_(False)
+    model.gemm_precision = getattr(args, "gemm_precision", "3xfp16")
+    os.makedirs(os.path.join(args.save_path, "in_the_wild"), exist_ok=True)
+    if rank == 0:
+        with open(os.path.join(args.save_path, "in_the_wild", "classes.json"), "w") as f:
+            json.dump({s: classes[s] for s in stems}, f, indent=1)
+    start, end = host.shard_range(len(stems), rank, world_size)
+    mine = stems[start:end]
+    for b0 in range(0, len(mine), args.batch_size):
+        batch = mine[b0:b0 + args.batch_size]
+        tic = time.perf_counter()
+        res = segment_images(model, [paths[s] for s in batch], [classes[s] for s in batch], img_size=args.img_size, drop_iter=args.drop_iter,
+                             threshold=args.threshold, postprocess=args.postprocess, max_att_block_num=args.max_att_block_num,
+                             prune_att_head=args.prune_att_head, data_type=data_type, batch_size=len(batch))
+        for s, r in zip(batch, res):
+            png, conf = wild_outputs(args.save_path, s)
+            write_label_png(png, r["ids"])
+            if r["conf"] is not None:
+                np.save(conf, r["conf"])
+        if rank == 0:
+            dt = time.perf_counter() - tic
+            print("Time: batch of %d images %.4f seconds (%.2f images/s on this rank)" % (len(batch), dt, len(batch) / dt))
+    if _fp16_range_exceeded(model, dev, 1):
+        print("warning: rank %d: an activation left fp16's range in a 3xFP16 GEMM operand; repeating its images with "
+              "--gemm_precision 3xtf32" % rank)
+        model.fp16_overflow_flag(dev).zero_()
+        args.gemm_precision = "3xtf32"
+        return main_in_the_wild(rank, world_size, args, model=model)
+    return mine
+
+
 def main(rank, world_size, args):
     from .blip_itm import BlipITM
+    if getattr(args, "in_the_wild", False):
+        return main_in_the_wild(rank, world_size, args)
     if getattr(args, "real_data", False):
         return main_real(rank, world_size, args)
     tic = time.perf_counter()

@@ -530,3 +530,27 @@ def confusion_accumulate(labels, gt, n_class, hist, lut=None, pred_out=None, bad
     check(_lib.load().pnp_confusion_accumulate(_p(labels), _p(gt), _p(lut), stride, _p(pred_out), _p(hist), _p(bad_count), B, N,
                                                int(n_class), _stream()), "pnp_confusion_accumulate")
     return hist
+
+
+def label_map(labels, lut, Q=None):
+    """ids[b,n] = lut[b, labels[b,n]] and, with the CRF marginals Q [B,N,Cp] of crf_inference, conf[b,n] = Q[b,n,labels[b,n]]
+    (pnp_label_map: the relabel of confusion_accumulate without ground truth).  A label outside [0, lut columns) gives id -1 and
+    conf -1.  labels int32 [B,N], lut int32 [B,C'] -> (ids int32 [B,N], conf float32 [B,N] or None)."""
+    _req(labels, torch.int32, "labels", 2)
+    _req(lut, torch.int32, "lut", 2)
+    B, N = labels.shape
+    if lut.shape[0] != B or lut.shape[1] < 1:
+        raise PnpError("lut must be [B, >=1]")
+    Cp = 0
+    if Q is not None:
+        _req(Q, torch.float32, "Q", 3)
+        if tuple(Q.shape[:2]) != (B, N) or Q.shape[2] < lut.shape[1]:
+            raise PnpError("Q must be [B,N,Cp] with Cp >= the lut's columns")
+        Cp = Q.shape[2]
+    ids = torch.empty((B, N), dtype=torch.int32, device=labels.device)
+    conf = torch.empty((B, N), dtype=torch.float32, device=labels.device) if Q is not None else None
+    if labels.numel() == 0:   # an empty tensor's null data pointer would read as a missing argument to the library
+        return ids, conf
+    check(_lib.load().pnp_label_map(_p(labels), _p(lut), lut.shape[1], _p(Q), Cp, _p(ids), _p(conf), B, N, _stream()),
+          "pnp_label_map")
+    return ids, conf

@@ -143,19 +143,21 @@ def postprocess_batch(class_maps, guides, gts, luts, hist, *, threshold, rescale
                       crf=None, bad_count=None, return_labels=False, stats=None, bilateral=None, n_classes=None):
     """class_maps [B,C,P,P] -> labels -> hist (accumulated in place).  guides uint8 [B,H,W,3]; gts float32 [B,H,W];
     luts int32 [B,C'] (composed relabel tables).  mode: the --postprocess string ('', 'blur', 'crf', 'blur+crf').
+    gts None (images without ground truth; hist is then unused): returns (ids int32 [B,H,W] relabelled through luts, conf float32
+    [B,H,W] = the CRF marginal of each chosen label, or None when the mode has no CRF) instead of counting anything.
     bilateral: a lattice already built over `guides` (the two reference passes of one batch share it).
     n_classes: int32 [B] CUDA tensor when the images have different class counts (class_maps padded to the largest; blurred modes
     only); luts then has Cp columns and the CRF runs over all Cp channels (the dead ones stay at Q = 0)."""
     B, C = class_maps.shape[:2]
     P_grid = class_maps.shape[-1]
-    H, W = gts.shape[1:]
+    H, W = (gts if gts is not None else guides).shape[1:3]
     N = H * W
     use_blur = bool(mode) and "blur" in mode
     use_crf = bool(mode) and "crf" in mode
     p = dict(CRF_DEFAULTS)
     p.update(crf or {})
     Cc = C + (1 if with_background else 0)
-    labels = U = None
+    labels = U = Q = None
     if n_classes is not None and not (use_blur and P_grid <= 32 and USE_LOWRANK_BLUR):
         raise PnpError("per-image class counts need the fused low-rank (d) group (a blurred mode, P <= 32)")
     if use_blur and P_grid <= 32 and USE_LOWRANK_BLUR:
@@ -185,8 +187,12 @@ def postprocess_batch(class_maps, guides, gts, luts, hist, *, threshold, rescale
         if stats is not None:
             stats["M_s"], stats["M_b"], stats["max_row_b"] = lat_s.M, lat_b.M, lat_b.struct.max_row
         _mark(stats, "lattice")
-        _, labels = ops.crf_inference([lat_s, lat_b], [p["pos_w"], p["bi_w"]], U, Cc, p["n_iter"], want_labels=True)
+        Q, labels = ops.crf_inference([lat_s, lat_b], [p["pos_w"], p["bi_w"]], U, Cc, p["n_iter"], want_labels=True)
         _mark(stats, "crf")
+    if gts is None:
+        ids, conf = ops.label_map(labels, luts, Q)
+        _mark(stats, "label_map")
+        return ids.view(B, H, W), (conf.view(B, H, W) if conf is not None else None)
     pred = torch.empty((B, N), dtype=torch.float32, device=labels.device) if return_labels else None
     ops.confusion_accumulate(labels, gts.view(B, N), n_class, hist, lut=luts, pred_out=pred, bad_count=bad_count)
     _mark(stats, "confusion")
@@ -260,6 +266,93 @@ def _side_stream(dev):
     return _SIDE_STREAMS[key]
 
 
+def _make_buckets(class_lists, dataset_ids, shapes, gts, guides, *, data_type, mode, patch_num, dev):
+    """Group the images of a batch by (channel key, background rule, (H, W) = shapes[b]) and upload each bucket's inputs.
+    Returns ({key: members}, {key: (gts [n,H,W] or None when gts is None, guides [n,H,W,3], composed relabel LUTs int32 [n,width])},
+    {key: (n_classes int32 [n] when the bucket's class counts differ, else None; largest class count)})."""
+    use_blur = bool(mode) and "blur" in mode
+    pad_classes = PAD_CLASSES_IN_BUCKETS and use_blur and patch_num <= 32 and USE_LOWRANK_BLUR
+    buckets = {}
+    for b in range(len(class_lists)):
+        C = len(class_lists[b])
+        with_bg = host.add_background_rule(data_type, C)
+        # with padded classes a bucket holds every class count that pads to the same Cp; else the exact count is part of the key
+        ckey = ops.crf_pad_channels(C + (1 if with_bg else 0)) if pad_classes else C
+        buckets.setdefault((ckey, with_bg, shapes[b]), []).append(b)
+    inputs, ncls = {}, {}
+    for key, members in buckets.items():
+        with_bg = key[1]
+        counts = [len(class_lists[b]) for b in members]
+        ragged_c = pad_classes and len(set(counts)) > 1
+        width = key[0] if ragged_c else counts[0] + (1 if with_bg else 0)     # LUT columns: Cp when the CRF runs over all of them
+        lut_rows = []
+        for b in members:
+            row = list(host.relabel_lut(dataset_ids[b], with_bg))
+            lut_rows.append(row + [0] * (width - len(row)))                    # dead channels are never the argmax
+        inputs[key] = (_as_device_batch(gts, members, torch.float32, dev) if gts is not None else None,
+                       _as_device_batch(guides, members, torch.uint8, dev), torch.tensor(lut_rows, dtype=torch.int32, device=dev))
+        ncls[key] = (torch.tensor(counts, dtype=torch.int32, device=dev), max(counts)) if ragged_c else (None, counts[0])
+    return buckets, inputs, ncls
+
+
+def _n_bucket_streams(buckets, dev):
+    """How many CUDA streams the buckets of a batch are spread over (0: everything on the current stream)."""
+    return min(int(BUCKET_STREAMS), len(buckets)) if (len(buckets) > 1 and dev.type == "cuda") else 0
+
+
+def _start_bucket_streams(dev, n_streams):
+    """The streams the buckets of a ragged batch are spread over (empty: everything on the current stream).  They start after
+    everything already enqueued on the current stream."""
+    if not n_streams:
+        return []
+    cur = torch.cuda.current_stream(dev)
+    pool = _bucket_streams(dev, n_streams)
+    for st in pool:
+        st.wait_stream(cur)
+    return pool
+
+
+def _join_bucket_streams(dev, pool):
+    if not pool:
+        return
+    cur = torch.cuda.current_stream(dev)
+    for st in pool:
+        cur.wait_stream(st)
+
+
+def _build_bucket_lattices(buckets, inputs, crf_p, dev, n_streams):
+    """{key: bilateral lattice over the bucket's guide images}, and the spatial lattice of every bucket shape cached."""
+    keys = list(buckets)
+    for key in keys:
+        _SPATIAL.get(key[2][0], key[2][1], crf_p["pos_xy_std"], dev)
+    pool = _start_bucket_streams(dev, n_streams)
+    # every build is enqueued before the first one is waited for (pnp_lattice_finish reads the vertex count back)
+    begun = _run_on_streams(dev, pool, [lambda key=key: ops.build_lattice_begin(key[2][0], key[2][1], crf_p["bi_xy_std"], rgb=inputs[key][1],
+                                                                                srgb=crf_p["bi_rgb_std"]) for key in keys])
+    done = _run_on_streams(dev, pool, [lambda lw=lw: ops.build_lattice_finish(*lw) for lw in begun])
+    _join_bucket_streams(dev, pool)
+    return dict(zip(keys, done))
+
+
+def _run_buckets(merged, buckets, ncls, dev, n_streams, one_bucket):
+    """one_bucket(key, class_maps) for every bucket, spread over the bucket streams; class_maps are the bucket's rows of the padded
+    token-merge output `merged`, cut to the bucket's largest class count.  Returns the results in bucket order."""
+    B = merged.shape[0]
+    pool = _start_bucket_streams(dev, n_streams)
+
+    def run(key, members):
+        c_max = ncls[key][1]
+        if len(members) == B and c_max == merged.shape[1]:
+            cm = merged
+        else:
+            cm = merged[torch.as_tensor(members, device=dev), :c_max].contiguous()
+        return one_bucket(key, cm)
+
+    out = _run_on_streams(dev, pool, [lambda key=key, members=members: run(key, members) for key, members in buckets.items()])
+    _join_bucket_streams(dev, pool)
+    return out
+
+
 def batch_confusion(gradcam_fn, imgs, token_ids, decode, class_lists, dataset_ids, gts, guides, *, drop_iter, patch_num,
                     threshold, data_type, mode, n_class, coco=False, crf=None, norm_imgs=None, stats=None, overlap=False,
                     labels_out=None, bad_count=None, defer=False):
@@ -300,29 +393,9 @@ def batch_confusion(gradcam_fn, imgs, token_ids, decode, class_lists, dataset_id
     _mark(stats, "start")
 
     # everything that depends on the inputs only: buckets, device copies, relabel LUTs, token segment tables
-    use_blur = bool(mode) and "blur" in mode
-    pad_classes = PAD_CLASSES_IN_BUCKETS and use_blur and patch_num <= 32 and USE_LOWRANK_BLUR
-    buckets = {}
-    for b in range(B):
-        C = len(class_lists[b])
-        with_bg = host.add_background_rule(data_type, C)
-        # with padded classes a bucket holds every class count that pads to the same Cp; else the exact count is part of the key
-        ckey = ops.crf_pad_channels(C + (1 if with_bg else 0)) if pad_classes else C
-        buckets.setdefault((ckey, with_bg, tuple(gts[b].shape)), []).append(b)
-    inputs, ncls = {}, {}
-    for key, members in buckets.items():
-        with_bg = key[1]
-        counts = [len(class_lists[b]) for b in members]
-        ragged_c = pad_classes and len(set(counts)) > 1
-        width = key[0] if ragged_c else counts[0] + (1 if with_bg else 0)     # LUT columns: Cp when the CRF runs over all of them
-        lut_rows = []
-        for b in members:
-            row = list(host.relabel_lut(dataset_ids[b], with_bg))
-            lut_rows.append(row + [0] * (width - len(row)))                    # dead channels are never the argmax
-        inputs[key] = (_as_device_batch(gts, members, torch.float32, dev), _as_device_batch(guides, members, torch.uint8, dev),
-                       torch.tensor(lut_rows, dtype=torch.int32, device=dev))
-        ncls[key] = (torch.tensor(counts, dtype=torch.int32, device=dev), max(counts)) if ragged_c else (None, counts[0])
-    n_streams = min(int(BUCKET_STREAMS), len(buckets)) if (len(buckets) > 1 and not timed_stages and dev.type == "cuda") else 0
+    buckets, inputs, ncls = _make_buckets(class_lists, dataset_ids, [tuple(gts[b].shape) for b in range(B)], gts, guides,
+                                          data_type=data_type, mode=mode, patch_num=patch_num, dev=dev)
+    n_streams = _n_bucket_streams(buckets, dev) if not timed_stages else 0
     segs = segment_tensors(token_ids, decode, class_lists, dev)
     hists = {}
     if round0_scored:
@@ -334,60 +407,26 @@ def batch_confusion(gradcam_fn, imgs, token_ids, decode, class_lists, dataset_id
     lattices = {}
     ev_lattices = None
 
-    def bucket_streams():
-        """The streams the buckets of a ragged batch are spread over (empty: everything on the current stream).  They start
-        after everything already enqueued on the current stream."""
-        if not n_streams:
-            return []
-        cur = torch.cuda.current_stream(dev)
-        pool = _bucket_streams(dev, n_streams)
-        for st in pool:
-            st.wait_stream(cur)
-        return pool
-
-    def join_streams(pool):
-        if not pool:
-            return
-        cur = torch.cuda.current_stream(dev)
-        for st in pool:
-            cur.wait_stream(st)
-
     def build_lattices():  # one bilateral lattice per bucket, shared by both passes (the guide images are the same)
         if use_crf:
-            keys = list(buckets)
-            for key in keys:
-                _SPATIAL.get(key[2][0], key[2][1], crf_p["pos_xy_std"], dev)
-            pool = bucket_streams()
-            # every build is enqueued before the first one is waited for (pnp_lattice_finish reads the vertex count back)
-            begun = _run_on_streams(dev, pool, [lambda key=key: ops.build_lattice_begin(key[2][0], key[2][1], crf_p["bi_xy_std"], rgb=inputs[key][1],
-                                                                                        srgb=crf_p["bi_rgb_std"]) for key in keys])
-            done = _run_on_streams(dev, pool, [lambda lw=lw: ops.build_lattice_finish(*lw) for lw in begun])
-            lattices.update(zip(keys, done))
-            join_streams(pool)
+            lattices.update(_build_bucket_lattices(buckets, inputs, crf_p, dev, n_streams))
             _mark(stats, "lattice")
 
     def run_pass(name, gmaps, rescale):
         merged = merge_tokens_batch(gmaps, token_ids, decode, class_lists, segs, padded=True)
         _mark(stats, "merge")
-        pool = bucket_streams()
 
-        def one_bucket(key, members):
+        def one_bucket(key, cm):
             gt, gd, lut = inputs[key]
-            n_cls, c_max = ncls[key]
-            if len(members) == B and c_max == merged.shape[1]:
-                cm = merged
-            else:
-                cm = merged[torch.as_tensor(members, device=dev), :c_max].contiguous()
             return postprocess_batch(cm, gd, gt, lut, hists[name], threshold=threshold, rescale=rescale, with_background=key[1],
                                      mode=mode, n_class=n_class, crf=crf, bad_count=bad, stats=stats, bilateral=lattices.get(key),
-                                     return_labels=labels_out is not None, n_classes=n_cls)
+                                     return_labels=labels_out is not None, n_classes=ncls[key][0])
 
         if labels_out is not None and len(buckets) != 1:
             raise PnpError("labels_out needs a uniform batch (one bucket)")
-        preds = _run_on_streams(dev, pool, [lambda key=key, members=members: one_bucket(key, members) for key, members in buckets.items()])
+        preds = _run_buckets(merged, buckets, ncls, dev, n_streams, one_bucket)
         if labels_out is not None:
             labels_out[name] = preds[0]
-        join_streams(pool)
 
     def side_prologue():
         """First use of the side stream for this batch: inputs visible, lattices built (under the running model pass)."""
@@ -436,6 +475,43 @@ def batch_confusion(gradcam_fn, imgs, token_ids, decode, class_lists, dataset_id
     if bad_count is None and int(bad.item()):
         raise PnpError("a relabelled id fell outside [0, n_class)")
     return hists.get("round0"), hists.get("all_drop"), chosen
+
+
+def batch_labels(gradcam_fn, imgs, token_ids, decode, class_lists, guides, *, drop_iter, patch_num, threshold, data_type, mode,
+                 crf=None, norm_imgs=None):
+    """The batch without ground truth: one label map per image, for images of any size and class list (the in-the-wild use).
+    Returns, in batch order, (ids int32 [H_b,W_b], conf float32 [H_b,W_b] or None) CUDA tensors at the size of each guide image:
+    ids 0 = background, i = class_lists[b][i-1]; conf = the CRF marginal of the chosen label (None when `mode` has no CRF).
+
+    The post-processed map is the one the reference scores: the accumulated map of the DropOut rounds when drop_iter > 1 (no
+    Scale_0_1 outside COCO, DRV:438 / DRVC:527), else the round-0 map (with Scale_0_1, DRV:362).  Buckets, streams, lattice
+    builds and post-processing are batch_confusion's, so each image's ids equal the relabelled map a batch of its own gives there.
+    imgs [B,3,S,S] cuda (modified in place by the DropOut rounds); guides: uint8 [H_b,W_b,3] arrays (list) or one CUDA tensor
+    [B,H,W,3]."""
+    dev = imgs.device
+    B = imgs.shape[0]
+    crf_p = dict(CRF_DEFAULTS)
+    crf_p.update(crf or {})
+    ids = [list(range(1, len(c) + 1)) for c in class_lists]
+    buckets, inputs, ncls = _make_buckets(class_lists, ids, [tuple(guides[b].shape[:2]) for b in range(B)], None, guides,
+                                          data_type=data_type, mode=mode, patch_num=patch_num, dev=dev)
+    n_streams = _n_bucket_streams(buckets, dev)
+    segs = segment_tensors(token_ids, decode, class_lists, dev)
+    g0, agg, _ = salience_dropout_loop(gradcam_fn, imgs, norm_imgs, drop_iter, patch_num)
+    lattices = _build_bucket_lattices(buckets, inputs, crf_p, dev, n_streams) if (bool(mode) and "crf" in mode) else {}
+    gmaps, rescale = (agg, data_type.startswith("coco")) if agg is not None else (g0, True)
+    merged = merge_tokens_batch(gmaps, token_ids, decode, class_lists, segs, padded=True)
+
+    def one_bucket(key, cm):
+        _, gd, lut = inputs[key]
+        return postprocess_batch(cm, gd, None, lut, None, threshold=threshold, rescale=rescale, with_background=key[1], mode=mode,
+                                 n_class=None, crf=crf, bilateral=lattices.get(key), n_classes=ncls[key][0])
+
+    out = [None] * B
+    for members, (ids_k, conf_k) in zip(buckets.values(), _run_buckets(merged, buckets, ncls, dev, n_streams, one_bucket)):
+        for j, b in enumerate(members):
+            out[b] = (ids_k[j], conf_k[j] if conf_k is not None else None)
+    return out
 
 
 def side_stream(dev):
